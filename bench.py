@@ -6,7 +6,7 @@ block of the chosen BASELINE config: K1a/K1b (re-order, wipe-off, forward FFT of
 (PRN x Doppler bin x block) correlation search with on-chip non-coherent accumulation, row peaks and
 the per-PRN decision.  cells = PRNs x Doppler bins x code phases (independent of K, SURVEY.md 8d).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1|2|3|4|5] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1|2|3|4|5] [--impl reference] [--dump-outputs DIR]
 
 Default workload: config 1, the Opensky-shaped block of BASELINE.json's north_star target.  The line carries
 `value` (device-resident input, CUDA events), `e2e` (N = 1: through gnssacq_search with a pageable host buffer,
@@ -19,6 +19,9 @@ pulled from rank 0 over NVLink by K1a, the candidates are stored into rank 0's t
 `--impl reference` times the CPU restatement of acquisition.m (oracle/, NumPy float64, literal 3-FFT
 loop) on all host cores, a FULL acquisition per step for configs 1 and 2: MATLAB/Octave do not exist in this
 image, so the oracle port is the reference arm (cpu_baseline.kind = "port").
+`--dump-outputs DIR` writes the result rows of the last timed step as DIR/<field>.npy (float64, one entry per PRN; the
+reference arm: prn and peak): the inputs are seeded, so two builds run with the same arguments can be compared output
+for output.
 """
 from __future__ import annotations
 
@@ -35,6 +38,7 @@ PKG = os.path.join(ROOT, "assignment-for-aae6102_gnss-sdr_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "search cells/s (PRN x Doppler x code-phase), 32-PRN acquisition"
 UNIT = "cells/s"
@@ -92,6 +96,22 @@ def synth_windows(cfg) -> list:
     from gnssacq.synth import opensky_recording, urban_recording
     rec = opensky_recording(seed=6102 + 1) if cfg["shape"] == "opensky" else urban_recording(seed=6102 + 2)
     return [rec.read(cfg["epoch_ms"] * j, cfg["k"] * cfg["m"]) for j in range(cfg["sweep_windows"])]
+
+
+# fields of gnssacq_result that the coarse search fills; fine_freq_hz stays NaN there (gnssacq_fine_frequency fills it)
+DUMP_FIELDS = ("prn", "acquired", "code_phase", "doppler_bin", "doppler_hz", "peak", "noise_meansq", "snr_db")
+
+
+def dump_outputs(directory, columns):
+    """--dump-outputs: one float64 array per output field (rows in PRN order) as <directory>/<field>.npy."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, values in columns.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(values, dtype=np.float64))
+
+
+def dump_rows(directory, rows):
+    dump_outputs(directory, {f: [getattr(r, f) for r in rows] for f in DUMP_FIELDS})
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -242,9 +262,12 @@ def run_reference(args, cfg):
         pool.map(_ref_worker, tasks, chunksize=1)
     t0 = time.perf_counter()
     for _ in range(n_steps):
-        pool.map(_ref_worker, tasks, chunksize=1)
+        peaks = pool.map(_ref_worker, tasks, chunksize=1)
     dt = time.perf_counter() - t0
     pool.close()
+    if args.dump_outputs:
+        # the per-PRN maximum of the surface over the first kb blocks (all of them when full_step is true)
+        dump_outputs(args.dump_outputs, {"prn": PRNS, "peak": peaks})
     scale = kb / cfg["k"]
     cells_per_step = len(PRNS) * cfg["bins"] * cfg["n"] * scale
     value = cells_per_step * n_steps / dt
@@ -393,6 +416,10 @@ def run_gpu(args, cfg):
             ev1[i].record()
         barrier()
         t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs:
+        timed_rows = shard.fetch()                          # the rows of the last timed step (rank 0 holds them)
+        if rank == 0:
+            dump_rows(args.dump_outputs, timed_rows)
     step_ms = [a.elapsed_time(b) for a, b in zip(ev0, ev1)]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -576,6 +603,8 @@ def run_gpu_epoch_sharded(args, cfg):
             s.enqueue_device(d_ifs[j % len(d_ifs)].data_ptr(), s.if_bytes)
             b.record()
         barrier()
+    if args.dump_outputs and mine and mine[-1] == args.steps - 1:    # the rank that searched the last epoch
+        dump_rows(args.dump_outputs, s.fetch())
     total_ms = torch.tensor([sum(a.elapsed_time(b) for a, b in ev)], dtype=torch.float64, device="cuda")
     # end to end: this rank's epochs straight from the recording file, one gnssacq_sweep_file call
     import tempfile
@@ -636,7 +665,11 @@ def main():
                     help="config 4 on N GPUs: shard every acquisition's PRN x Doppler grid (default, BASELINE's wording) or deal out the epochs")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of the timed result")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result rows of the last timed step as DIR/<field>.npy (float64, one entry per PRN)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)
