@@ -109,7 +109,9 @@ __global__ void finalize_kernel(const Candidate* __restrict__ cand, int P, int B
 // out[ms][rho][m] = sample 16*m + rho of that ms (see Wipe2Args).  Input is read with 16-byte vector loads
 // (8 packed int8 I/Q samples per load, fully coalesced) -- `raw` may be a PEER pointer: on ranks > 0 of a
 // multi-GPU search this kernel is what pulls the IF block out of rank 0's HBM over NVLink, so no separate
-// broadcast is needed.  A CTA handles TM consecutive m of one ms (TM*16 samples, contiguous in the input).
+// broadcast is needed.  Until the root's "IF ready" flag, which this kernel waits for, that buffer holds whatever it
+// held before (the previous block, a half-finished upload), so nothing else on such a rank reads `raw`: the int16
+// means are summed from the comb copy.  A CTA handles TM consecutive m of one ms (TM*16 samples, contiguous in the input).
 constexpr int kCombTM = 256;
 // Flags of the multi-GPU exchange live in the ROOT GPU's memory; other GPUs read / write them over NVLink.
 __device__ __forceinline__ void flag_store_sys(unsigned* p, unsigned v) {
@@ -176,7 +178,9 @@ __global__ void xchg_wait_kernel(const unsigned* done_flags, int world, unsigned
     if ((has_rows >> r) & 1ull) flag_wait_sys(done_flags + r, epoch, timeout);
 }
 
-// acquisition.m:30-32 -- per-component mean of the int16 I/Q block (exact integer sums).
+// acquisition.m:30-32 -- per-component mean of the int16 I/Q block (exact integer sums).  On the comb-row path the
+// sums scan the handle's comb copy, i.e. the block as pulled (its zero pad pairs included), on the K1 v1 path the IF
+// block itself; means_kernel divides by the true sample count N*K*M either way.
 __global__ void sum_int16_kernel(const int16_t* __restrict__ s, long long n_pairs, long long* __restrict__ sums) {
     long long si = 0, sq = 0;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_pairs;
@@ -1052,16 +1056,16 @@ static int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out = 
     auto& xc = h->xc;
     if (xchg && !h->d_comb) return fail(h, GNSSACQ_ERR_STATE, "the multi-GPU exchange needs the comb-row K1 (shared memory too small for this shape)");
     CU(cudaEventRecord(h->ev[1], s));
-    const double* means = nullptr;
-    if (h->cfg.data_precision == 2) {
-        const long long pairs = (long long)h->N * h->K * h->M;
+    // int16 (acquisition.m:30-32): per-component means of the N*K*M samples, from `scan` (I, Q) pairs at `src`
+    const double* means = h->cfg.data_precision == 2 ? h->d_means : nullptr;
+    auto launch_means = [&](const void* src, long long scan) -> int {
         CU(cudaMemsetAsync(h->d_sums, 0, 2 * sizeof(long long), s));
-        sum_int16_kernel<<<296, 256, 0, s>>>((const int16_t*)d_if, pairs, h->d_sums);
-        means_kernel<<<1, 1, 0, s>>>(h->d_sums, pairs, h->d_means);
+        sum_int16_kernel<<<296, 256, 0, s>>>((const int16_t*)src, scan, h->d_sums);
+        means_kernel<<<1, 1, 0, s>>>(h->d_sums, (long long)h->N * h->K * h->M, h->d_means);
         CU(cudaGetLastError());
         h->launches += 2;
-        means = h->d_means;
-    }
+        return GNSSACQ_OK;
+    };
     if (h->d_comb) {
         const int bps = h->cfg.data_type * h->cfg.data_precision;
         const int rows = h->N / 16, tiles = (rows + kCombTM - 1) / kCombTM;
@@ -1072,6 +1076,11 @@ static int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out = 
             xchg ? xc.flags + 63 : nullptr);
         CU(cudaGetLastError());
         if (xchg) CU(cudaEventRecord(xc.ev_b, s));
+        // from the comb copy, not `d_if`: on a non-root shard that is the root's buffer (see comb_kernel).
+        // [K*M*16 rows][pitch bytes], one (I, Q) pair per 4 bytes; the pad bytes are zero (memset at create, never written)
+        if (means) {
+            if (int rc = launch_means(h->d_comb, (long long)h->K * h->M * 16 * h->comb_pitch / 4)) return rc;
+        }
         Wipe2Args w2;
         w2.comb = h->d_comb;
         w2.pitch = h->comb_pitch;
@@ -1084,6 +1093,10 @@ static int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out = 
         CU(h->ops->launch_wipe2(w2, (int)h->base_freq.size() * h->K, s));
         h->launches += 2;
     } else {
+        // (K1 v1 is never used by the multi-GPU exchange: `d_if` is this handle's own, complete block)
+        if (means) {
+            if (int rc = launch_means(d_if, (long long)h->N * h->K * h->M)) return rc;
+        }
         WipeArgs wa;
         wa.raw = d_if;
         wa.data_type = h->cfg.data_type;

@@ -84,6 +84,26 @@ def oracle_rows_chunked(raw_bytes, file, signal, acq, prns, *, coh_ms=1, chunk_b
     return [peak_and_snr(surf[p], signal, acq, p) for p in prns]
 
 
+def assert_fine_frequency_matches(got, longraw, file, signal, acq, sats):
+    """acquisition.m:83-127's fineFreq of every SV of `sats` (`got`, from the GPU) against the oracle on `longraw`
+    ((L+1) ms as read by :89-100).  Index exact unless the oracle's two best spectral lines are within the FP32 tie
+    tolerance; for I/Q data the line must also be the carrier, IF + the satellite's Doppler."""
+    n, L, datalen = int(signal.Sample), int(acq.L), int(acq.datalen)
+    res = signal.Fs / (L * n * datalen)
+    for sat, g in zip(sats, got):
+        want, idx, pk, runner = oracle.fine_frequency(longraw, file, signal, acq, sat.prn, sat.codedelay, detail=True)
+        if runner >= pk * (1.0 - 1e-5):             # magnitude tie (|.|, i.e. half the relative gap of power)
+            # real input: |X[k]| == |X[F-k]| exactly, so the reference's first-max over the WHOLE spectrum
+            # (acquisition.m:116 searches 1:2*halffftlength) is decided by rounding; accept the mirror line too
+            mirror = (L * n * datalen - idx + 2) * res if file.dataType == 1 else want
+            assert min(abs(g - want), abs(g - mirror)) <= res * 1.0001, (sat.prn, g, want, mirror)
+        else:
+            assert g == want, (sat.prn, g, want, idx)
+        # and it is the carrier: within two 5 Hz-class bins of IF + true Doppler (incl. the 1-based-index quirk)
+        if file.dataType == 2:
+            assert abs((g - signal.IF) - sat.doppler_hz) <= max(3 * res, 1e3 / L), (sat.prn, g)
+
+
 def assert_rows_match(gpu_rows, ref_rows, *, thr=12.0, what=""):
     """BASELINE.json north_star: peak metric and SNR within 1e-4 relative for EVERY row; code phase, Doppler bin
     and the decision bit-exact unless the oracle's own top two cells are closer than TIE_TOL (then FP32 may

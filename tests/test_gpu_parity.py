@@ -14,7 +14,7 @@ from oracle.acquisition_ref import correlation_surface
 from oracle.synth import SatSpec, VirtualFile, synth_if, urban_spec, opensky_spec
 import gnssacq
 from gnssacq import api
-from helpers import structs, small_spec, oracle_rows, assert_rows_match, METRIC_RTOL
+from helpers import structs, small_spec, oracle_rows, assert_rows_match, assert_fine_frequency_matches, METRIC_RTOL
 
 pytestmark = pytest.mark.gpu
 import ctypes as _C
@@ -233,19 +233,7 @@ def test_fine_frequency_stage(fs, if_hz, data_type, precision, datalen):
         with pytest.raises(gnssacq.GnssAcqError) as e:
             s.fine_frequency(raw_long[:-2], L, prns, cds)
         assert e.value.code == -3
-    res = fs / (L * n * datalen)
-    for prn, cd, g, sat in zip(prns, cds, got, sats):
-        want, idx, pk, runner = oracle.fine_frequency(longraw, file, signal, acq, prn, cd, detail=True)
-        if runner >= pk * (1.0 - 1e-5):             # magnitude tie (|.|, i.e. half the relative gap of power)
-            # real input: |X[k]| == |X[F-k]| exactly, so the reference's first-max over the WHOLE spectrum
-            # (acquisition.m:116 searches 1:2*halffftlength) is decided by rounding; accept the mirror line too
-            mirror = (L * n * datalen - idx + 2) * res if data_type == 1 else want
-            assert min(abs(g - want), abs(g - mirror)) <= res * 1.0001, (prn, g, want, mirror)
-        else:
-            assert g == want, (prn, g, want, idx)
-        # and it is the carrier: within two 5 Hz-class bins of IF + true Doppler (incl. the 1-based-index quirk)
-        if data_type == 2:
-            assert abs((g - if_hz) - sat.doppler_hz) <= max(3 * res, 1e3 / L), (prn, g)
+    assert_fine_frequency_matches(got, longraw, file, signal, acq, sats)
 
 
 def test_wrapper_fills_fine_freq():
