@@ -144,15 +144,23 @@ struct gnssacq_handle {
     gnss::DevPtr<gnssacq_result> d_res;
     gnss::DevPtr<float> d_surface;
     gnss::DevPtr<gnss::cf> d_scratch;
+    int xmode = 1;                 // exchange: 1 = DSMEM, 2 = L2 + persistent clusters, 3 = L2 + cooperative CTA groups
+    // schedule of the current row set (use_schedule in gnssacq.cu); d_scratch, d_group_ctr, d_row_slots hold group_cap groups
     int l2x_clusters = 0;          // > 0: use the L2-exchange persistent search kernel with this many clusters
     int coop_groups = 0;           // > 0: use the cluster-free cooperative kernel with this many CTA groups
+    bool by_blocks = false;        // cooperative kernel: block-granular tail (needs d_partial)
+    int group_cap = 0;
     gnss::DevPtr<unsigned> d_group_ctr;
     int bin0 = 0, B_full = 0;      // this handle's bins are [bin0, bin0 + B) of the B_full-bin grid
-    int row0 = 0, n_rows = 0;      // ... and of that P x B grid (row = bin * P + prn index) it searches rows [row0, row0 + n_rows)
+    int row0 = 0, n_rows = 0;      // ... and of that P x B grid (row = bin * P + prn index) it searches rows [row0, row0 + n_rows),
+    bool windows = false;          // ... or, with Doppler windows set, the n_rows rows listed in d_rows
+    gnss::DevPtr<int> d_rows;      // [P*B] grid row ids inside the windows, bin-major (built by the first gnssacq_set_doppler_windows)
+    int used_groups = 0, used_split = 1;   // schedule of the last enqueued search (gnssacq_stats)
     gnss::Xchg xc;
     const gnssacq_result* d_last_rows = nullptr;   // where the last enqueued search wrote its rows (d_res or the caller's buffer)
     gnss::DevPtr<gnss::Candidate> d_row_slots;
     gnss::DevPtr<float> d_partial;         // cooperative kernel: accumulators of row parts handed between groups
+    int partial_groups = 0;                // ... for this many groups (0: not built yet)
     gnss::DevPtr<long long> d_sums;
     gnss::DevPtr<double> d_means;
     std::unique_ptr<gnss::FftState> fft;

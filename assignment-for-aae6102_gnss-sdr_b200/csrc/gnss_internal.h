@@ -22,7 +22,10 @@ struct SearchArgs {
     const int* bin_base;   // [B] which base a bin derives from
     const int* bin_shift;  // [B] shift in FFT bins relative to that base (SURVEY A.7)
     int P, B, K;
-    int row_first, n_rows; // this launch searches rows [row_first, +n_rows) of the grid, row = b*P + p (all of them: 0, P*B)
+    int row_first, n_rows; // this launch searches rows [row_first, +n_rows) of the grid, row = b*P + p (all of them: 0, P*B) ...
+    const int* rows;       // ... or, when not null, the n_rows grid rows listed here, bin-major (Doppler windows).  The
+                           // contiguous range is computed, not looked up: a per-row table read on the path to the next
+                           // row's first loads cost the default search kernels 1 % (B200, configs 1 and 2)
     int w;                 // ceil(Fs/fc) (acquisition.m:66)
     Candidate* cand;       // [P][cand_stride]: row (p, b) at cand[p*cand_stride + b].  A shard of a multi-GPU search
                            // points this straight into the ROOT GPU's table (peer memory, NVLink stores)

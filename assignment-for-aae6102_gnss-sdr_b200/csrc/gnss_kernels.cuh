@@ -368,7 +368,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel(SearchArgs a) {
     float* acc = reinterpret_cast<float*>(D + S::D_ELEMS);
     Tw4* tw = reinterpret_cast<Tw4*>(acc + Smem<Q, R>::acc_floats);
     RedScratch* rs = reinterpret_cast<RedScratch*>(tw + 100);
-    const int row = a.row_first + unit;         // row = bin * P + prn_index (PRN fastest: rows in
+    const int row = a.rows ? a.rows[unit] : a.row_first + unit;   // row = bin * P + prn_index (PRN fastest: rows in
     const int p = row % a.P, b = row / a.P;     // flight share the same forward spectra in L2)
 
     fill_tw125(tw, tid, T);
@@ -472,7 +472,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
     PowerAccumStorer st{acc};
 
     for (int lrow = slot; lrow < a.n_rows; lrow += ncl) {
-        const int row = a.row_first + lrow;
+        const int row = a.rows ? a.rows[lrow] : a.row_first + lrow;
         const int p = row % a.P, b = row / a.P;
         for (int e = tid; e < S::ACC_ELEMS; e += T) acc[e] = 0.f;
         int sa, sb, sc;
@@ -723,9 +723,9 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
             }
         }
     };
-    const int n_rows = a.n_rows;              // the handle's rows are [row_first, row_first + n_rows) of the P x B grid
-    auto loader_of = [&](int lrow) {          // loader of block 0 of a row (two dependent table reads: once per row)
-        const int row = a.row_first + lrow;
+    const int n_rows = a.n_rows;              // the launch's rows: a.rows[0 .. n_rows), or [row_first, row_first + n_rows)
+    auto loader_of = [&](int lrow) {          // loader of block 0 of a row (two or three dependent table reads: once per row)
+        const int row = a.rows ? a.rows[lrow] : a.row_first + lrow;
         const int p = row % a.P, b = row / a.P;
         int sa, sb, sc;
         G::shift_coords(a.bin_shift[b], sa, sb, sc);
@@ -884,7 +884,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
                                       a.K - cp.ke, tid);
                 __syncthreads();
             }
-            const int p = (a.row_first + row) % a.P, b = (a.row_first + row) / a.P;
+            const int grow = a.rows ? a.rows[row] : a.row_first + row, p = grow % a.P, b = grow / a.P;
             float bv = -1.f;
             int bm = INT_MAX;
             double ss = 0.0;

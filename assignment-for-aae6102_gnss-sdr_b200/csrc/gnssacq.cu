@@ -263,9 +263,78 @@ void fill_engine_stats(const gnssacq_handle* h, gnssacq_stats* st) {
     st->n_bases = (int)h->base_freq.size();
     st->cluster_ctas = h->ops->R;
     st->threads = h->ops->T;
-    st->exchange = h->coop_groups > 0 ? 3 : (h->l2x_clusters > 0 ? 2 : 1);
-    st->resident_clusters = h->coop_groups > 0 ? h->coop_groups : h->l2x_clusters;
-    st->work_split = h->d_partial ? 2 : 1;
+    st->exchange = h->xmode;
+    st->resident_clusters = h->used_groups;
+    st->work_split = h->used_split;
+}
+
+// How the persistent search kernels (exchange 2 / 3) deal out one row set: the resident groups, and whether the
+// cooperative kernel hands the tail out block by block.  Chosen per row set: at create for the handle's own rows, and
+// again for every set of Doppler windows (160 rows on 37 groups want the block tail where 1 312 rows do not).
+struct Schedule { int groups = 0; bool by_blocks = false; };
+
+// Exchange 2 / 3: `n` groups made resident, but never more than there is work for.  The cooperative kernel deals out
+// single blocks of a row (block-granular tail) or whole rows; the clustered one whole rows.
+// Block-granular tail (see search_kernel_coop): needs K-1 power planes per group (150 MB at the reference's sizes) --
+// not possible above 2 GiB or beyond the kernel's 32-bit unit arithmetic.  It costs 0.15-0.4 row times (publishing and
+// adding the planes), so work_split 0 (auto) uses it only where whole rows would leave >= 4 % of the last round's
+// group-time idle (measured r01: pays for <= 8 PRNs at N = 26 000, <= 4 PRNs at N = 58 000, not for 32).  Results are
+// identical either way.  rows == 0: nothing to launch.
+int plan_schedule(gnssacq_handle* h, long long rows, Schedule& sc) {
+    sc = Schedule{};
+    if (h->xmode == 1 || rows == 0) return GNSSACQ_OK;
+    const VariantOps* ops = h->ops;
+    const int split = h->cfg.work_split;
+    int n = h->xmode == 3 ? ops->max_groups_coop() : ops->max_clusters_l2x();
+    bool by_blocks = h->xmode == 3 && split != 1 && h->K > 1 && (unsigned long long)n * n * h->K < (1ull << 32) &&
+                     (unsigned long long)n * (h->K - 1) * ops->partial_bytes_per_group <= (2ull << 30);
+    if (by_blocks && split == 0) {
+        const long long rounds = (rows + n - 1) / n;
+        by_blocks = (double)(rounds * n - rows) >= 0.04 * (double)(rounds * n);
+    }
+    const long long max_useful = by_blocks ? rows * h->K : rows;
+    if (n > max_useful) n = (int)max_useful;
+    if (n <= 0) return fail(h, GNSSACQ_ERR_CUDA, "persistent search kernel cannot be made resident on this device");
+    sc.groups = n;
+    sc.by_blocks = by_blocks;
+    return GNSSACQ_OK;
+}
+
+// Makes `sc` the handle's schedule.  Per-group buffers are only ever grown, and the hand-over planes are built the
+// first time a schedule asks for the block-granular tail; what is built goes into the handle only once every call
+// has succeeded, so a failure leaves the previous schedule whole.  Any search still using the old buffers must have
+// finished (create: none yet; gnssacq_set_doppler_windows waits for the stream).
+int use_schedule(gnssacq_handle* h, const Schedule& sc) {
+    const VariantOps* ops = h->ops;
+    const size_t n = (size_t)sc.groups;
+    DevPtr<cf> scratch;
+    DevPtr<unsigned> ctr;
+    DevPtr<Candidate> slots;
+    DevPtr<float> partial;
+    const bool grow = sc.groups > h->group_cap;
+    if (grow) {
+        CU(alloc(scratch, n * ops->scratch_bytes_per_cluster), GNSSACQ_ERR_NOMEM);
+        // the padding columns of the exchange layout are never written: they must read as exact zeros
+        CU(cudaMemsetAsync(scratch.get(), 0, n * ops->scratch_bytes_per_cluster, h->stream), GNSSACQ_ERR_NOMEM);
+        CU(alloc(ctr, n * (2 + ops->R) * sizeof(unsigned)), GNSSACQ_ERR_NOMEM);     // group barriers + hand-over counters + row tickets
+        CU(alloc(slots, n * ops->R * sizeof(Candidate)), GNSSACQ_ERR_NOMEM);
+    }
+    const bool planes = sc.by_blocks && sc.groups > h->partial_groups;
+    if (planes) CU(alloc(partial, n * (h->K - 1) * ops->partial_bytes_per_group), GNSSACQ_ERR_NOMEM);
+    if (grow) {
+        h->d_scratch = std::move(scratch);
+        h->d_group_ctr = std::move(ctr);
+        h->d_row_slots = std::move(slots);
+        h->group_cap = sc.groups;
+    }
+    if (planes) {
+        h->d_partial = std::move(partial);
+        h->partial_groups = sc.groups;
+    }
+    h->coop_groups = h->xmode == 3 ? sc.groups : 0;
+    h->l2x_clusters = h->xmode == 2 ? sc.groups : 0;
+    h->by_blocks = sc.by_blocks;
+    return GNSSACQ_OK;
 }
 
 const VariantOps* pick_variant(int Q, int R, int T) {
@@ -307,6 +376,17 @@ void plan_bins(gnssacq_handle* h) {
         h->bin_base[b] = found;
         h->bin_shift[b] = shift;
     }
+}
+
+// For a handle that does not search all of its P x B rows: the cells of its candidate table that no search writes must
+// not win K4's maximum (peak -1 never does), and the rows of the kept surface that it never searches read as zeros.
+// Synchronous (the sentinel table is a temporary).
+int clear_unsearched(gnssacq_handle* h) {
+    std::vector<Candidate> none((size_t)h->P * h->B, Candidate{-1.f, 0, 0.0, 0.0});
+    CU(cudaMemcpyAsync(h->d_cand.get(), none.data(), none.size() * sizeof(Candidate), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
+    if (h->d_surface) CU(cudaMemsetAsync(h->d_surface.get(), 0, (size_t)h->P * h->B * h->N * sizeof(float), h->stream), GNSSACQ_ERR_NOMEM);
+    CU(cudaStreamSynchronize(h->stream), GNSSACQ_ERR_NOMEM);
+    return GNSSACQ_OK;
 }
 
 int validate(const gnssacq_config* c, std::string& why) {
@@ -456,6 +536,7 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
     sa.bin_shift = h->d_bin_shift.get();
     sa.P = h->P; sa.B = h->B; sa.K = h->K;
     sa.row_first = h->row0; sa.n_rows = h->n_rows;
+    sa.rows = h->windows ? h->d_rows.get() : nullptr;
     sa.w = h->w;
     sa.cand = xchg ? xc.cand_all + (size_t)xc.sh.prn_first * xc.sh.freq_num_total + xc.sh.bin_first : h->d_cand.get();
     sa.cand_stride = xchg ? xc.sh.freq_num_total : h->B;
@@ -466,7 +547,7 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
     sa.partial = h->d_partial.get();
     sa.part_ctr = h->d_group_ctr ? h->d_group_ctr.get() + h->coop_groups : nullptr;
     sa.row_ticket = h->d_group_ctr ? h->d_group_ctr.get() + (size_t)h->coop_groups * (1 + h->ops->R) : nullptr;
-    sa.row_granular = h->d_partial ? 0 : 1;
+    sa.row_granular = h->by_blocks ? 0 : 1;
 #ifdef GNSS_TIMELINE
     static unsigned long long* d_timeline = nullptr;
     if (!d_timeline) { CU(cudaMalloc(&d_timeline, 16 * 16 * 32 * sizeof(unsigned long long))); }
@@ -474,15 +555,19 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
     sa.timeline = d_timeline;
     g_timeline = d_timeline;
 #endif
-    if (h->coop_groups > 0) {
-        CU(cudaMemsetAsync(h->d_group_ctr.get(), 0, (size_t)h->coop_groups * (2 + h->ops->R) * sizeof(unsigned), s));
-        CU(h->ops->launch_search_coop(sa, h->coop_groups, s));
-    } else if (h->l2x_clusters > 0) {
-        CU(h->ops->launch_search_l2x(sa, h->l2x_clusters, s));
-    } else {
-        CU(h->ops->launch_search(sa, h->n_rows, s));
+    h->used_groups = h->coop_groups + h->l2x_clusters;
+    h->used_split = h->by_blocks ? 2 : 1;
+    if (h->n_rows > 0) {                   // (0: Doppler windows that hold no bin; K4 reports every PRN as not searched)
+        if (h->coop_groups > 0) {
+            CU(cudaMemsetAsync(h->d_group_ctr.get(), 0, (size_t)h->coop_groups * (2 + h->ops->R) * sizeof(unsigned), s));
+            CU(h->ops->launch_search_coop(sa, h->coop_groups, s));
+        } else if (h->l2x_clusters > 0) {
+            CU(h->ops->launch_search_l2x(sa, h->l2x_clusters, s));
+        } else {
+            CU(h->ops->launch_search(sa, h->n_rows, s));
+        }
+        h->launches += 1;
     }
-    h->launches += 1;
     CU(cudaEventRecord(h->ev[3].get(), s));
     if (xchg) {
         // candidates went straight into the root's table; a non-root shard now raises its "done" flag there,
@@ -722,36 +807,14 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     CU(alloc(h->d_means, 2 * sizeof(double)), GNSSACQ_ERR_NOMEM);
     // exchange: 1 = DSMEM clusters, 2 = L2 buffer + clusters, 3 = L2 buffer + cooperative groups (no clusters).
     // auto: cooperative groups for the two real front ends (fastest measured, profiles/r01), DSMEM for tiny N.
-    const int xmode = cfg->exchange ? cfg->exchange : (Q >= 13 ? 3 : 1);
-    if (xmode == 2 || xmode == 3) {
-        int n = xmode == 3 ? ops->max_groups_coop() : ops->max_clusters_l2x();
-        // the cooperative kernel deals out single blocks of a row (work_split 0) or whole rows (1); the
-        // clustered one whole rows
-        // Block-granular tail (see search_kernel_coop): needs K-1 power planes per group (150 MB at the
-        // reference's sizes) -- not possible above 2 GiB or beyond the kernel's 32-bit unit arithmetic.  It
-        // costs 0.15-0.4 row times (publishing and adding the planes), so work_split 0 (auto) uses it only
-        // where whole rows would leave >= 4 % of the last round's group-time idle (measured r01: pays for
-        // <= 8 PRNs at N = 26 000, <= 4 PRNs at N = 58 000, not for 32).  Results are identical either way.
-        bool by_blocks = xmode == 3 && cfg->work_split != 1 && h->K > 1 && (unsigned long long)n * n * h->K < (1ull << 32) &&
-                         (unsigned long long)n * (h->K - 1) * ops->partial_bytes_per_group <= (2ull << 30);
-        if (by_blocks && cfg->work_split == 0) {
-            const long long rows = h->n_rows, rounds = (rows + n - 1) / n;
-            by_blocks = (double)(rounds * n - rows) >= 0.04 * (double)(rounds * n);
-        }
-        const long long max_useful = by_blocks ? (long long)h->n_rows * h->K : (long long)h->n_rows;
-        if (n > max_useful) n = (int)max_useful;
-        if (n <= 0) return fail(nullptr, GNSSACQ_ERR_CUDA, "persistent search kernel cannot be made resident on this device");
-        if (xmode == 3) h->coop_groups = n; else h->l2x_clusters = n;
-        CU(alloc(h->d_scratch, (size_t)n * ops->scratch_bytes_per_cluster), GNSSACQ_ERR_NOMEM);
-        // the padding columns of the exchange layout are never written: they must read as exact zeros
-        CU(cudaMemsetAsync(h->d_scratch.get(), 0, (size_t)n * ops->scratch_bytes_per_cluster, h->stream), GNSSACQ_ERR_NOMEM);
-        CU(alloc(h->d_group_ctr, (size_t)n * (2 + ops->R) * sizeof(unsigned)), GNSSACQ_ERR_NOMEM);     // group barriers + hand-over counters + row tickets
-        if (by_blocks) CU(alloc(h->d_partial, (size_t)n * (h->K - 1) * ops->partial_bytes_per_group), GNSSACQ_ERR_NOMEM);
-        CU(alloc(h->d_row_slots, (size_t)n * ops->R * sizeof(Candidate)), GNSSACQ_ERR_NOMEM);
+    h->xmode = cfg->exchange ? cfg->exchange : (Q >= 13 ? 3 : 1);
+    {
+        Schedule sc;
+        if (int rc = plan_schedule(h, h->n_rows, sc)) return rc;
+        if (int rc = use_schedule(h, sc)) return rc;
     }
     if (cfg->keep_surface) {
         CU(alloc(h->d_surface, (size_t)h->P * h->B * N * sizeof(float)), GNSSACQ_ERR_NOMEM);
-        if (h->n_rows < h->P * h->B) CU(cudaMemsetAsync(h->d_surface.get(), 0, (size_t)h->P * h->B * N * sizeof(float), h->stream), GNSSACQ_ERR_NOMEM);   // rows it never searches read as zeros
     }
     CU(alloc(h->h_if, h->if_bytes), GNSSACQ_ERR_NOMEM);
     CU(alloc(h->h_res, h->P * sizeof(gnssacq_result)), GNSSACQ_ERR_NOMEM);
@@ -763,11 +826,8 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     CU(cudaMemcpyAsync(h->d_bin_shift.get(), h->bin_shift.data(), h->B * sizeof(int), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
     CU(cudaMemcpyAsync(h->d_prn.get(), cfg->prn, h->P * sizeof(int), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
     CU(cudaMemcpyAsync(h->d_base_freq.get(), h->base_freq.data(), nb * sizeof(double), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
-    if (h->n_rows < h->P * h->B) {
-        // a row range: the cells of the handle's own table that it never writes must not win K4's maximum
-        std::vector<Candidate> none((size_t)h->P * h->B, Candidate{-1.f, 0, 0.0, 0.0});
-        CU(cudaMemcpyAsync(h->d_cand.get(), none.data(), none.size() * sizeof(Candidate), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
-        CU(cudaStreamSynchronize(h->stream), GNSSACQ_ERR_NOMEM);
+    if (h->n_rows < h->P * h->B) {                              // a row range
+        if (int rc = clear_unsearched(h)) return rc;
     }
     std::vector<double> bw(nb);                                 // (read by a copy that the final sync waits for)
     {
@@ -801,6 +861,40 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
 int gnssacq_set_stream(gnssacq_handle* h, void* s) {
     if (!h) return GNSSACQ_ERR_INVALID_ARG;
     h->stream = (s == GNSSACQ_OWN_STREAM) ? h->own_stream.get() : (cudaStream_t)s;
+    return GNSSACQ_OK;
+}
+
+// The windows only choose which rows of the full grid K2 walks: the forward spectra, K1 and the int16 means are the
+// full grid's, so a windowed PRN's candidates are bit for bit those of the full search in its window's bins, and K4
+// over a table whose other cells hold the peak -1 sentinel picks what a bin_first / bin_count handle would.
+int gnssacq_set_doppler_windows(gnssacq_handle* h, const double* lo_hz, const double* hi_hz) {
+    if (!h) return GNSSACQ_ERR_INVALID_ARG;
+    if (!lo_hz != !hi_hz) return fail(h, GNSSACQ_ERR_INVALID_ARG, "lo_hz and hi_hz must both be given or both be NULL");
+    if (lo_hz) {
+        for (int i = 0; i < h->P; ++i)
+            if (!(lo_hz[i] <= hi_hz[i])) return fail(h, GNSSACQ_ERR_INVALID_ARG, "a Doppler window has lo_hz > hi_hz or a NaN bound");
+    }
+    if (h->cfg.bin_count > 0 || h->cfg.row_count > 0) return fail(h, GNSSACQ_ERR_STATE, "Doppler windows need a handle over the full grid (bin_count = row_count = 0)");
+    if (h->xc.on) return fail(h, GNSSACQ_ERR_STATE, "Doppler windows are not available in the multi-GPU exchange");
+    // grid row ids, bin-major: the strided schedule then keeps the groups on neighbouring rows (the same forward spectra).
+    // Cleared: all P*B rows, which the search kernels walk without the list.
+    std::vector<int> rows;
+    rows.reserve((size_t)h->P * h->B);
+    for (int b = 0; b < h->B; ++b) {
+        const double f = std::fma(h->cfg.freq_step_hz, (double)b, h->cfg.freq_min_hz);   // K4's doppler_hz (a fused multiply-add there)
+        for (int p = 0; p < h->P; ++p)
+            if (!lo_hz || (lo_hz[p] <= f && f <= hi_hz[p])) rows.push_back(b * h->P + p);
+    }
+    CU(cudaSetDevice(h->device));
+    CU(cudaStreamSynchronize(h->stream));                       // an enqueued search may still read the old tables
+    if (lo_hz && !h->d_rows) CU(alloc(h->d_rows, (size_t)h->P * h->B * sizeof(int)), GNSSACQ_ERR_NOMEM);
+    Schedule sc;
+    if (int rc = plan_schedule(h, (long long)rows.size(), sc)) return rc;
+    if (int rc = use_schedule(h, sc)) return rc;
+    if (lo_hz) CU(cudaMemcpyAsync(h->d_rows.get(), rows.data(), rows.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    if (int rc = clear_unsearched(h)) return rc;                // (synchronises: `rows` is a temporary)
+    h->n_rows = (int)rows.size();
+    h->windows = lo_hz != nullptr;
     return GNSSACQ_OK;
 }
 

@@ -118,6 +118,7 @@ EXPORTS = (
     "gnssacq_loop_params_default", "gnssacq_track",
     "gnssacq_shard_plan", "gnssacq_shard_plan_rows", "gnssacq_xchg_root", "gnssacq_xchg_attach", "gnssacq_xchg_attach_local",
     "gnssacq_xchg_if_buffer", "gnssacq_xchg_enqueue", "gnssacq_xchg_finish", "gnssacq_xchg_fetch",
+    "gnssacq_set_doppler_windows",
 )
 
 
@@ -165,6 +166,7 @@ def _load() -> C.CDLL:
     lib.gnssacq_xchg_finish.argtypes = [vp]
     lib.gnssacq_xchg_fetch.argtypes = [vp, C.POINTER(Result), C.POINTER(Stats)]
     lib.gnssacq_fp32_peak_tflops.argtypes = [C.c_int32, C.POINTER(C.c_double)]
+    lib.gnssacq_set_doppler_windows.argtypes = [vp, vp, vp]
     return lib
 
 
@@ -306,6 +308,19 @@ class Searcher:
 
     def set_stream(self, cuda_stream: int) -> None:
         self._check(lib.gnssacq_set_stream(self._h, C.c_void_p(cuda_stream)))
+
+    def set_doppler_windows(self, lo_hz: Sequence[float], hi_hz: Sequence[float]) -> None:
+        """Search PRN i (cfg.prn order) only over the grid bins whose Doppler lies in [lo_hz[i], hi_hz[i]], for every
+        later search until :meth:`clear_doppler_windows`.  A PRN whose window holds no bin is not searched."""
+        lo = np.ascontiguousarray(lo_hz, dtype=np.float64)
+        hi = np.ascontiguousarray(hi_hz, dtype=np.float64)
+        if lo.shape != (self.cfg.n_prn,) or hi.shape != (self.cfg.n_prn,):
+            raise ValueError(f"need {self.cfg.n_prn} lower and upper bounds")
+        self._check(lib.gnssacq_set_doppler_windows(self._h, lo.ctypes.data, hi.ctypes.data))
+
+    def clear_doppler_windows(self) -> None:
+        """Search the full grid again."""
+        self._check(lib.gnssacq_set_doppler_windows(self._h, None, None))
 
     def search(self, if_bytes) -> List[Result]:
         """Host buffer in (bytes / bytearray / numpy int8|int16), result rows out."""

@@ -20,6 +20,11 @@
  *   cfg.n_gpus   (default 1)  number of GPUs the PRN list is sharded over (PRN-major, SURVEY 8e): the gateway
  *                             keeps one handle per GPU and 'search' goes through gnssacq_search_multi
  *   cfg.devices  (optional)   the CUDA device ordinals to use, numel >= n_gpus (default 0 .. n_gpus-1)
+ *   cfg.doppler_lo_hz, cfg.doppler_hi_hz  (optional, 'search' and 'sweep_file', both or neither)  n_prn-element
+ *                             per-PRN Doppler windows (gnssacq_set_doppler_windows): PRN cfg.prn(i) is searched only
+ *                             over the grid bins with doppler_lo_hz(i) <= doppler_hz <= doppler_hi_hz(i); a PRN whose
+ *                             window holds no bin comes back with acquired 0, snr_db NaN, peak -1.  Left out: the
+ *                             full grid
  * 'search' returns an n_prn x 8 double matrix, one row per searched PRN, in the order of cfg.prn:
  *   [prn acquired code_phase doppler_bin doppler_hz peak noise_meansq snr_db]
  * ('sweep_file': n_prn x 8 x n).  The handles are kept in statics between calls (mexLock) and rebuilt only when
@@ -40,7 +45,7 @@ static gnssacq_handle* g_handle[MAX_GPUS];
 static int g_n_handles = 0;
 static gnssacq_config g_cfg;
 static int g_gpus = 0, g_dev[MAX_GPUS];
-static int g_have_cfg = 0, g_locked = 0;
+static int g_have_cfg = 0, g_locked = 0, g_windows = 0;
 
 static void close_all(void) {
     int i;
@@ -48,6 +53,7 @@ static void close_all(void) {
         if (g_handle[i]) { gnssacq_destroy(g_handle[i]); g_handle[i] = NULL; }
     g_n_handles = 0;
     g_have_cfg = 0;
+    g_windows = 0;
 }
 
 static double field(const mxArray* s, const char* name, double dflt) {
@@ -146,9 +152,35 @@ static void ensure_handles(const mxArray* cs, gnssacq_config* cfg_out) {
     *cfg_out = c;
 }
 
+/* cfg.doppler_lo_hz / cfg.doppler_hi_hz -> every handle's slice of the windows (PRN-major shards, as in
+ * ensure_handles); neither field: clear windows an earlier call set */
+static void apply_windows(const mxArray* cs, const gnssacq_config* c) {
+    const mxArray* lo = mxGetField(cs, 0, "doppler_lo_hz");
+    const mxArray* hi = mxGetField(cs, 0, "doppler_hi_hz");
+    int g, rc;
+    if (!lo && !hi) {
+        for (g = 0; g_windows && g < g_n_handles; ++g) {
+            rc = gnssacq_set_doppler_windows(g_handle[g], NULL, NULL);
+            if (rc != GNSSACQ_OK) fail(rc, gnssacq_last_error(g_handle[g]));
+        }
+        g_windows = 0;
+        return;
+    }
+    if (!lo || !hi || !mxIsDouble(lo) || !mxIsDouble(hi) || (int)mxGetNumberOfElements(lo) != c->n_prn ||
+        (int)mxGetNumberOfElements(hi) != c->n_prn)
+        fail(GNSSACQ_ERR_INVALID_ARG, "cfg.doppler_lo_hz and cfg.doppler_hi_hz must both be double with n_prn elements");
+    g_windows = 1;
+    for (g = 0; g < g_n_handles; ++g) {
+        const int first = g * c->n_prn / g_n_handles;
+        rc = gnssacq_set_doppler_windows(g_handle[g], mxGetPr(lo) + first, mxGetPr(hi) + first);
+        if (rc != GNSSACQ_OK) fail(rc, gnssacq_last_error(g_handle[g]));
+    }
+}
+
 void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     static const char* usage =
-        "usage: gnssacq_mex(mode, ...), mode = 'search' | 'fine' | 'sweep_file' | 'track_load' | 'correlate' | 'track' | 'close'";
+        "usage: gnssacq_mex(mode, ...), mode = 'search' | 'fine' | 'sweep_file' | 'track_load' | 'correlate' | 'track' | 'close'"
+        " ('search' and 'sweep_file' take optional per-PRN windows cfg.doppler_lo_hz / cfg.doppler_hi_hz)";
     char mode[24];
     gnssacq_config c;
     size_t nbytes;
@@ -163,6 +195,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     if (strcmp(mode, "search") == 0) {                 /* acquisition.m:41-80 */
         gnssacq_result* rows;
         if (nrhs != 3 || !(mxIsInt8(prhs[1]) || mxIsInt16(prhs[1]))) fail(GNSSACQ_ERR_INVALID_ARG, "search: raw must be int8 or int16");
+        apply_windows(prhs[2], &c);
         rows = (gnssacq_result*)mxMalloc(sizeof(gnssacq_result) * (size_t)c.n_prn);
         rc = (g_n_handles == 1) ? gnssacq_search(g_handle[0], mxGetData(prhs[1]), nbytes, rows, NULL)
                                 : gnssacq_search_multi(g_handle, g_n_handles, mxGetData(prhs[1]), nbytes, rows);
@@ -198,6 +231,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         n_win = (int)mxGetScalar(prhs[5]);
         if (n_win < 1) fail(GNSSACQ_ERR_INVALID_ARG, "sweep_file: n_windows >= 1");
         if (g_n_handles != 1) fail(GNSSACQ_ERR_INVALID_ARG, "sweep_file runs on one GPU (cfg.n_gpus = 1)");
+        apply_windows(prhs[2], &c);
         rows = (gnssacq_result*)mxMalloc(sizeof(gnssacq_result) * (size_t)c.n_prn * (size_t)n_win);
         rc = gnssacq_sweep_file(g_handle[0], path, (int64_t)mxGetScalar(prhs[3]), (int32_t)mxGetScalar(prhs[4]), n_win, rows, NULL);
         if (rc != GNSSACQ_OK) { mxFree(rows); fail(rc, gnssacq_last_error(g_handle[0])); }

@@ -178,6 +178,19 @@ int gnssacq_search_multi(gnssacq_handle* const* hs, int32_t n_handles, const voi
 int gnssacq_sweep(gnssacq_handle* h, const void* const* windows, int32_t n_windows, size_t nbytes_each,
                   gnssacq_result* out, gnssacq_stats* stats);
 
+/* Assisted re-acquisition: per-PRN Doppler windows for every later search on this handle (gnssacq_search,
+ * _search_device, _enqueue_device[_out], _search_multi, _sweep, _sweep_file) until cleared.  lo_hz[i] / hi_hz[i]
+ * belong to cfg.prn[i]; PRN i is searched over the bins b of the handle's grid with
+ * lo_hz[i] <= freq_min_hz + freq_step_hz*b <= hi_hz[i] (the doppler_hz K4 reports).  Only those rows are searched, so
+ * the search time follows the number of bins in the windows, not freq_num.  A windowed PRN's row is byte-identical to
+ * the row of a one-PRN handle with bin_first / bin_count set to its window's bins (doppler_bin / doppler_hz on this
+ * handle's full grid); the int16 means stay those of the whole block.  A PRN whose window holds no bin is not searched:
+ * its row has acquired = 0, snr_db = NaN, peak = -1.  lo_hz == hi_hz == NULL clears the windows (full grid again).
+ * lo_hz > hi_hz, a NaN bound or exactly one NULL array: GNSSACQ_ERR_INVALID_ARG.  A handle made with bin_count or
+ * row_count, or in the multi-GPU exchange: GNSSACQ_ERR_STATE (and gnssacq_xchg_root / _attach / _attach_local refuse
+ * a handle with windows set).  Synchronous: waits for the handle's stream and returns once the tables are in HBM. */
+int gnssacq_set_doppler_windows(gnssacq_handle* h, const double* lo_hz, const double* hi_hz);
+
 /* ---- one acquisition sharded over several GPUs, exchange through peer memory (no NCCL in the step) -------------
  * SURVEY 8e.  The (PRN, Doppler bin) rows of ONE acquisition are dealt out to `world` handles, one per GPU
  * (processes or one process): whole PRNs per shard when n_prn >= world, otherwise every shard takes all PRNs and a
