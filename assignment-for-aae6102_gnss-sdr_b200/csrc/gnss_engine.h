@@ -550,40 +550,149 @@ struct FineLoader {
     int start;                           // 0-based first sample = N - codedelay - 1 (acquisition.m:106)
     int L, n2, r;
     long long F;                         // fftlength = L*N*datalen (acquisition.m:108)
+    // decimated sample n1 (of N), code-stripped and modulated for residue r
+    GNSS_HD cf sample(int n1) const {
+        const long long n = (long long)L * n1 + n2;
+        const long long idx = (long long)start + n;
+        float xi, xq;
+        if (precision == 2) {
+            const int16_t* p = (const int16_t*)raw;
+            xi = (float)p[2 * idx] - mean_i;
+            xq = (float)p[2 * idx + 1] - mean_q;
+        } else if (data_type == 2) {
+            const int8_t* p = (const int8_t*)raw;
+            xi = (float)p[2 * idx];
+            xq = (float)p[2 * idx + 1];
+        } else {
+            xi = (float)((const int8_t*)raw)[idx];
+            xq = 0.f;
+        }
+        const float cv = (float)ca[chip[n]];
+        xi *= cv;
+        xq *= cv;
+        const long long m = (n * (long long)r) % F;          // exact phase numerator
+        const double fr = (double)m / (double)F;
+        float co, si;
+#if defined(__CUDA_ARCH__)
+        sincospif((float)(2.0 * fr), &si, &co);
+#else
+        co = (float)cos(2.0 * 3.14159265358979323846 * fr);
+        si = (float)sin(2.0 * 3.14159265358979323846 * fr);
+#endif
+        // (xi + i xq) * (co - i si)
+        return mk(xi * co + xq * si, xq * co - xi * si);
+    }
     template <int Q>
     GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
         static_for<0, Q>([&](auto c_) {
             constexpr int C = decltype(c_)::value;
-            const int n1 = Geo<Q>::good(a, b, C);
-            const long long n = (long long)L * n1 + n2;
-            const long long idx = (long long)start + n;
-            float xi, xq;
-            if (precision == 2) {
-                const int16_t* p = (const int16_t*)raw;
-                xi = (float)p[2 * idx] - mean_i;
-                xq = (float)p[2 * idx + 1] - mean_q;
-            } else if (data_type == 2) {
-                const int8_t* p = (const int8_t*)raw;
-                xi = (float)p[2 * idx];
-                xq = (float)p[2 * idx + 1];
-            } else {
-                xi = (float)((const int8_t*)raw)[idx];
-                xq = 0.f;
+            z[C] = sample(Geo<Q>::good(a, b, C));
+        });
+    }
+};
+
+// ---- zero-padded shapes: each ms of n_ms < N samples is the start of an N-point transform ----
+// K1 (acquisition.m:43,56): WipeoffLoader with the fold's stride and the sample count per ms taken at run time;
+// inputs n >= n_ms are the zero padding.  The carrier phase is that of sample j*n_ms + n + 1 of the coherent block.
+struct PadWipeoffLoader {
+    static constexpr bool kStreams = false;
+    const void* __restrict__ raw;   // start of this coherent block
+    int data_type, precision, coh_ms;
+    int n_ms;                       // samples per ms
+    double f_hz, fs_hz;
+    float mean_i, mean_q;
+    template <int Q>
+    GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
+        static_for<0, Q>([&](auto c_) {
+            constexpr int C = decltype(c_)::value;
+            const int n = Geo<Q>::good(a, b, C);
+            float ax = 0.f, ay = 0.f;
+            if (n < n_ms) {
+                for (int j = 0; j < coh_ms; ++j) {
+                    const long long idx = (long long)j * n_ms + n;
+                    float xi, xq;
+                    if (precision == 2) {
+                        const int16_t* p = (const int16_t*)raw;
+                        xi = (float)p[2 * idx] - mean_i;
+                        xq = (float)p[2 * idx + 1] - mean_q;
+                    } else if (data_type == 2) {
+                        const int8_t* p = (const int8_t*)raw;
+                        xi = (float)p[2 * idx];
+                        xq = (float)p[2 * idx + 1];
+                    } else {
+                        xi = (float)((const int8_t*)raw)[idx];
+                        xq = 0.f;
+                    }
+                    float co, si;
+                    carrier_sincos(f_hz, fs_hz, idx + 1, co, si);
+                    ax += xi * co - xq * si;
+                    ay += xi * si + xq * co;
+                }
             }
-            const float cv = (float)ca[chip[n]];
-            xi *= cv;
-            xq *= cv;
-            const long long m = (n * (long long)r) % F;          // exact phase numerator
-            const double fr = (double)m / (double)F;
-            float co, si;
-#if defined(__CUDA_ARCH__)
-            sincospif((float)(2.0 * fr), &si, &co);
-#else
-            co = (float)cos(2.0 * 3.14159265358979323846 * fr);
-            si = (float)sin(2.0 * 3.14159265358979323846 * fr);
-#endif
-            // (xi + i xq) * (co - i si)
-            z[C] = mk(xi * co + xq * si, xq * co - xi * si);
+            z[C] = mk(ax, ay);
+        });
+    }
+};
+
+// Bluestein stage 1: a[n] = x[n] * conj(ch[n]) for n < n, zero beyond.  `Src` gives x[n] through sample(n).
+struct NaturalSource {
+    const cf* __restrict__ in;
+    GNSS_HD cf sample(int n) const { return in[n]; }
+};
+template <class Src>
+struct ChirpLoader {
+    static constexpr bool kStreams = false;
+    Src src;
+    const cf* __restrict__ chirp;
+    int n;
+    template <int Q>
+    GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
+        static_for<0, Q>([&](auto c_) {
+            constexpr int C = decltype(c_)::value;
+            const int m = Geo<Q>::good(a, b, C);
+            if (m < n) {
+                const cf v = src.sample(m), c = chirp[m];
+                z[C] = mk(v.x * c.x + v.y * c.y, v.y * c.x - v.x * c.y);       // v * conj(c)
+            } else {
+                z[C] = mk(0.f, 0.f);
+            }
+        });
+    }
+};
+// Bluestein stage 2 input: conj(FFT(a) * H)
+struct ConjProdLoader {
+    static constexpr bool kStreams = false;
+    const cf* __restrict__ v;
+    const cf* __restrict__ filt;
+    template <int Q>
+    GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
+        static_for<0, Q>([&](auto c_) {
+            constexpr int C = decltype(c_)::value;
+            const int m = Geo<Q>::good(a, b, C);
+            const cf p = cmul_scalar(v[m], filt[m]);
+            z[C] = mk(p.x, -p.y);
+        });
+    }
+};
+// Bluestein stage 2 output W: X[k] = conj(ch[k] * W[k]) / N' for k < n, natural order; k >= n is dropped
+struct ChirpStorer {
+    cf* __restrict__ out;
+    const cf* __restrict__ chirp;
+    int n;
+    float scale;                    // 1 / N'
+    GNSS_HD void put(int k, cf w) {
+        if (k < n) {
+            const cf p = cmul_scalar(chirp[k], w);
+            out[k] = mk(p.x * scale, -p.y * scale);
+        }
+    }
+    template <int Q, int R>
+    GNSS_HD void store2(int col, int, const cf (&w0)[16], const cf (&w1)[16]) {
+        static_for<0, 16>([&](auto i_) {
+            constexpr int I = decltype(i_)::value;
+            constexpr int AP = (I / 4) + 4 * (I % 4);
+            put(Geo<Q>::lag_of(AP, col), w0[I]);
+            if (col + 1 < Geo<Q>::ROW) put(Geo<Q>::lag_of(AP, col + 1), w1[I]);
         });
     }
 };

@@ -93,12 +93,13 @@ struct FineState {
     DevPtr<void> raw;
     DevPtr<uint16_t> chip;
     DevPtr<cf> u;
+    DevPtr<cf> v;                          // padded shapes: [chunk][K][L][NF] first Bluestein stage
     DevPtr<int8_t> ca;
     DevPtr<int> start;
     DevPtr<unsigned long long> best;
 };
 
-struct FftState { DevPtr<cf> in, out; };
+struct FftState { DevPtr<cf> in, out, v; };      // v: padded shapes, [NF] first Bluestein stage
 
 // multi-GPU exchange (gnssacq_xchg_*): set up complete or not at all
 struct Xchg {
@@ -126,6 +127,7 @@ struct gnssacq_handle {
     const gnss::VariantOps* ops = nullptr;
     int device = 0;
     int N = 0, P = 0, B = 0, K = 0, M = 0;
+    int NF = 0;                            // transform length: N for a built N, else the built length each ms is zero-padded into
     int w = 0;
     size_t if_bytes = 0;
     std::vector<int> bin_base, bin_shift;
@@ -135,6 +137,7 @@ struct gnssacq_handle {
     gnss::DevPtr<int8_t> d_scode;
     gnss::DevPtr<gnss::cf> d_cc;
     gnss::DevPtr<gnss::cf> d_x;
+    gnss::DevPtr<gnss::cf> d_chirp, d_chirp_filt;   // padded shapes: Bluestein tables ch [N] and H [NF] (gnss::ChirpArgs)
     gnss::DevPtr<int> d_bin_base, d_bin_shift, d_prn;
     gnss::DevPtr<double> d_base_freq;
     gnss::DevPtr<double> d_base_w;         // (IF + doppler) / Fs per base, cycles per sample (K1 v2)
@@ -199,6 +202,8 @@ int cuda_fail(gnssacq_handle* h, cudaError_t e, const char* call, int oom_code =
         if (e__ != cudaSuccess) return ::gnss::cuda_fail(h, e__, #call, ##__VA_ARGS__);                  \
     } while (0)
 
+// transform length for `n` samples per ms (n itself, or the built length it is zero-padded into), 0: unsupported
+int transform_length(int n);
 // GNSSACQ_OK, or the status for an invalid config with the reason in `why`
 int validate(const gnssacq_config* c, std::string& why);
 

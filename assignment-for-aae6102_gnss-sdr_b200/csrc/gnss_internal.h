@@ -27,10 +27,12 @@ struct SearchArgs {
                            // contiguous range is computed, not looked up: a per-row table read on the path to the next
                            // row's first loads cost the default search kernels 1 % (B200, configs 1 and 2)
     int w;                 // ceil(Fs/fc) (acquisition.m:66)
+    int n_lags;            // lags a row reports: samples per ms.  The transform length for a built N; less for a handle that
+                           // zero-pads each ms into a longer transform, whose lags >= n_lags are not part of the correlation
     Candidate* cand;       // [P][cand_stride]: row (p, b) at cand[p*cand_stride + b].  A shard of a multi-GPU search
                            // points this straight into the ROOT GPU's table (peer memory, NVLink stores)
     int cand_stride;       // >= B (the full grid's bin count when the handle owns a bin sub-range)
-    float* surface;        // optional [P][B][N] (debug), lag order
+    float* surface;        // optional [P][B][n_lags] (debug), lag order
     cf* scratch;           // L2-exchange variants: [groups][2][16][RS] (double-buffered finished rows)
     unsigned* group_ctr;   // coop variant: one arrival counter per CTA group (zeroed before the launch)
     Candidate* row_slots;  // coop variant: [groups][R] per-CTA partial row results
@@ -47,6 +49,7 @@ struct WipeArgs {
     const void* raw;       // device IF block
     int data_type, precision, coh_ms, K;
     size_t block_bytes;    // bytes per coherent block
+    int n_ms;              // samples per ms (the fold's stride); < N: wipe_pad_kernel zero-pads each ms to the transform length
     const double* base_freq_hz;   // [n_bases] IF + doppler of each base
     double fs_hz;
     const double* means;   // [2] int16 path (device), else nullptr
@@ -90,6 +93,19 @@ struct FineArgs {
     cf* u;                       // [n_sv][K][L][N] natural order
 };
 
+// Bluestein (chirp-z) N-point DFTs, for an N that is not a built transform length, through the built N'-point
+// engine (N' >= 2N-1):  X[k] = conj(ch[k]) * (a (*) h)[k],  a[n] = x[n] conj(ch[n]) zero-padded to N',
+// ch[n] = exp(i pi n^2 / N), h the chirp filter ch[j], |j| < N, wrapped mod N'.  The circular convolution is
+// conj(FFT(conj(FFT(a) * H))) / N' with H = FFT(h), built once per handle.
+struct ChirpArgs {
+    const cf* chirp;       // [n] ch[n]
+    const cf* filt;        // [N'] H, natural order
+    int n;                 // DFT length N
+    const cf* in;          // [units][n] natural-order input (chirp_in_kernel; the fine stage loads its own)
+    cf* v;                 // [units][N'] FFT(a), natural order
+    cf* out;               // [units][n] X, natural order
+};
+
 struct VariantOps {
     int Q, R, T;
     size_t smem_search, smem_transform;
@@ -109,6 +125,11 @@ struct VariantOps {
     cudaError_t (*launch_search_coop)(const SearchArgs&, int groups, cudaStream_t);
     int (*max_groups_coop)();              // co-resident CTA groups on the current device
     size_t partial_bytes_per_group;        // coop variant: one power plane (all R slices) of the tail hand-over
+    // zero-padded shapes (samples per ms < N): K1 gather kernel, and the three stages of a Bluestein DFT
+    cudaError_t (*launch_wipe_pad)(const WipeArgs&, int units, cudaStream_t);
+    cudaError_t (*launch_chirp_in)(const ChirpArgs&, int units, cudaStream_t);       // ChirpArgs.in -> v
+    cudaError_t (*launch_fine_chirp)(const FineArgs&, const ChirpArgs&, int units, cudaStream_t);   // fine samples -> v
+    cudaError_t (*launch_chirp_out)(const ChirpArgs&, int units, cudaStream_t);      // v -> out
 };
 
 // defined in gnss_q3.cu / gnss_q13.cu / gnss_q29.cu

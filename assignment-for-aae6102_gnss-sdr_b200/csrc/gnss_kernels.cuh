@@ -6,6 +6,7 @@
 //                      load stage, transform, |.|^2, accumulate on chip; then K3 = row peak, first-index
 //                      argmax, sum of squares and windowed sum of squares   (acquisition.m:59,62-63,67)
 //   natural_kernel     plain forward DFT (test hook)
+//   wipe_pad_kernel, chirp_*_kernel   K1 and the Bluestein N-point DFTs of a shape zero-padded into the transform
 //
 // One transform = one thread-block cluster of R CTAs; each CTA keeps 16/R rows of the
 // [16][Q][125] prime-factor array in shared memory, pass 4 pulls the other CTAs' rows through
@@ -362,6 +363,79 @@ __global__ void __launch_bounds__(T, MINB) fine_kernel(FineArgs a) {
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
 
+// ---- zero-padded shapes (samples per ms < N) ----
+// K1 for a padded shape: wipe_kernel with the fold stride and the zero padding of PadWipeoffLoader
+template <int Q, int R, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) wipe_pad_kernel(WipeArgs a) {
+    GNSS_KERNEL_PROLOGUE
+    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
+    fill_tw125(tw, tid, T);
+    __syncthreads();
+    const int base = unit / a.K, k = unit - base * a.K;
+    PadWipeoffLoader ld;
+    ld.raw = (const unsigned char*)a.raw + (size_t)k * a.block_bytes;
+    ld.data_type = a.data_type;
+    ld.precision = a.precision;
+    ld.coh_ms = a.coh_ms;
+    ld.n_ms = a.n_ms;
+    ld.f_hz = a.base_freq_hz[base];
+    ld.fs_hz = a.fs_hz;
+    ld.mean_i = a.means ? (float)a.means[0] : 0.f;
+    ld.mean_q = a.means ? (float)a.means[1] : 0.f;
+    SpectrumStorer st{a.x + (size_t)unit * G::NX, 1.0f, 0, 1};
+    unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
+}
+
+// Bluestein stage 1 of gnssacq_fft_forward: v[unit] = FFT_N(conj(ch) * in[unit], zero-padded)
+template <int Q, int R, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) chirp_in_kernel(ChirpArgs c) {
+    GNSS_KERNEL_PROLOGUE
+    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
+    fill_tw125(tw, tid, T);
+    __syncthreads();
+    ChirpLoader<NaturalSource> ld{NaturalSource{c.in + (size_t)unit * c.n}, c.chirp, c.n};
+    NaturalStorerHD st{c.v + (size_t)unit * G::N};
+    unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
+}
+
+// Bluestein stage 1 of the fine stage: the samples of fine_kernel's unit ((sv * K) + r) * L + n2, chirped and padded
+template <int Q, int R, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) fine_chirp_kernel(FineArgs a, ChirpArgs c) {
+    GNSS_KERNEL_PROLOGUE
+    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
+    fill_tw125(tw, tid, T);
+    __syncthreads();
+    const int n2 = unit % a.L, r = (unit / a.L) % a.K, sv = unit / (a.L * a.K);
+    FineLoader f;
+    f.raw = a.raw;
+    f.chip = a.chip;
+    f.ca = a.ca + (size_t)sv * 1023;
+    f.data_type = a.data_type;
+    f.precision = a.precision;
+    f.mean_i = a.means ? (float)a.means[0] : 0.f;
+    f.mean_q = a.means ? (float)a.means[1] : 0.f;
+    f.start = a.start[sv];
+    f.L = a.L;
+    f.n2 = n2;
+    f.r = r;
+    f.F = a.F;
+    ChirpLoader<FineLoader> ld{f, c.chirp, c.n};
+    NaturalStorerHD st{c.v + (size_t)unit * G::N};
+    unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
+}
+
+// Bluestein stage 2: out[unit] = conj(ch * FFT_N(conj(v[unit] * H))) / N, first n outputs
+template <int Q, int R, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) chirp_out_kernel(ChirpArgs c) {
+    GNSS_KERNEL_PROLOGUE
+    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
+    fill_tw125(tw, tid, T);
+    __syncthreads();
+    ConjProdLoader ld{c.v + (size_t)unit * G::N, c.filt};
+    ChirpStorer st{c.out + (size_t)unit * c.n, c.chirp, c.n, 1.0f / (float)G::N};
+    unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
+}
+
 template <int Q, int R, int T, int MINB>
 __global__ void __launch_bounds__(T, MINB) search_kernel(SearchArgs a) {
     GNSS_KERNEL_PROLOGUE
@@ -394,12 +468,12 @@ __global__ void __launch_bounds__(T, MINB) search_kernel(SearchArgs a) {
     for (int e = tid; e < S::ACC_ELEMS; e += T) {
         const int ap = e / S::CH, t = e - ap * S::CH;
         const int col = rank * S::CH + t;
-        if (col < S::ROW) {
+        const int m = G::lag_of(ap, col);
+        if (col < S::ROW && m < a.n_lags) {         // (m >= n_lags: zero padding of a padded shape)
             const float v = acc[e];
-            const int m = G::lag_of(ap, col);
             if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
             ss += (double)v * (double)v;
-            if (a.surface) a.surface[((size_t)p * a.B + b) * G::N + m] = v;
+            if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
         }
     }
     block_reduce<T>(bv, bm, ss, rs);
@@ -422,7 +496,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel(SearchArgs a) {
     double wsum = 0.0;
     for (int i = tid; i < 2 * a.w - 1; i += T) {
         const int m = gm - (a.w - 1) + i;
-        if (m >= 0 && m < G::N) {
+        if (m >= 0 && m < a.n_lags) {
             int ap, col;
             G::cell_of_lag(m, ap, col);
             if (col / S::CH == rank) {
@@ -529,12 +603,12 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
         for (int e = tid; e < S::ACC_ELEMS; e += T) {
             const int ap = e / S::CH, t = e - ap * S::CH;
             const int col = rank * S::CH + t;
-            if (col < S::ROW) {
+            const int m = G::lag_of(ap, col);
+            if (col < S::ROW && m < a.n_lags) {         // (m >= n_lags: zero padding of a padded shape)
                 const float v = acc[e];
-                const int m = G::lag_of(ap, col);
                 if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
                 ss += (double)v * (double)v;
-                if (a.surface) a.surface[((size_t)p * a.B + b) * G::N + m] = v;
+                if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
             }
         }
         block_reduce<T>(bv, bm, ss, rs);
@@ -557,7 +631,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
         double wsum = 0.0;
         for (int i = tid; i < 2 * a.w - 1; i += T) {
             const int m = gm - (a.w - 1) + i;
-            if (m >= 0 && m < G::N) {
+            if (m >= 0 && m < a.n_lags) {
                 int ap, col;
                 G::cell_of_lag(m, ap, col);
                 if (col / S::CH == rank) {
@@ -888,16 +962,18 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
             float bv = -1.f;
             int bm = INT_MAX;
             double ss = 0.0;
-            if (a.surface) {                       // debug path: every cell's lag is needed anyway
+            if (a.surface || a.n_lags < G::N) {   // debug path and padded shapes: every cell's lag is needed
                 for (int e = tid; e < SX::ACC_ELEMS; e += T) {
                     const int ap = e / SX::CHX, t = e - ap * SX::CHX;
                     const int ex = rank * SX::CHX + t;
                     if (GX::valid(ex)) {
-                        const float v = acc[e];
                         const int m = GX::lag_of(ap, ex);
-                        if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
-                        ss += (double)v * (double)v;
-                        a.surface[((size_t)p * a.B + b) * G::N + m] = v;
+                        if (m < a.n_lags) {        // (m >= n_lags: zero padding of a padded shape)
+                            const float v = acc[e];
+                            if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
+                            ss += (double)v * (double)v;
+                            if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
+                        }
                     }
                 }
             } else {
@@ -947,7 +1023,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
             double wsum = 0.0;
             for (int i = tid; i < 2 * a.w - 1; i += T) {
                 const int m = gm - (a.w - 1) + i;
-                if (m >= 0 && m < G::N) {
+                if (m >= 0 && m < a.n_lags) {
                     int ap, ex;
                     GX::cell_of_lag(m, ap, ex);
                     if (ex / SX::CHX == rank) {
@@ -1036,6 +1112,14 @@ struct Variant {
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(fine_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
         if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(wipe_pad_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(chirp_in_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(fine_chirp_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(chirp_out_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
+        if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(search_kernel_coop<Q, R, T, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, R>::search);
         if (e != cudaSuccess) return e;
 
@@ -1094,6 +1178,32 @@ struct Variant {
     static cudaError_t launch_fine(const FineArgs& a, int units, cudaStream_t s) {
         return launch_clustered(fine_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
     }
+    static cudaError_t launch_wipe_pad(const WipeArgs& a, int units, cudaStream_t s) {
+        return launch_clustered(wipe_pad_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
+    }
+    static cudaError_t launch_chirp_in(const ChirpArgs& c, int units, cudaStream_t s) {
+        return launch_clustered(chirp_in_kernel<Q, RT, TT, MT>, c, units, RT, TT, Smem<Q, RT>::transform, s);
+    }
+    static cudaError_t launch_fine_chirp(const FineArgs& a, const ChirpArgs& c, int units, cudaStream_t s) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)(units * RT), 1, 1);
+        cfg.blockDim = dim3((unsigned)TT, 1, 1);
+        cfg.dynamicSmemBytes = Smem<Q, RT>::transform;
+        cfg.stream = s;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = (unsigned)RT;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
+        FineArgs fa = a;
+        ChirpArgs ca = c;
+        return cudaLaunchKernelEx(&cfg, fine_chirp_kernel<Q, RT, TT, MT>, fa, ca);
+    }
+    static cudaError_t launch_chirp_out(const ChirpArgs& c, int units, cudaStream_t s) {
+        return launch_clustered(chirp_out_kernel<Q, RT, TT, MT>, c, units, RT, TT, Smem<Q, RT>::transform, s);
+    }
     static cudaError_t launch_search(const SearchArgs& a, int rows, cudaStream_t s) {
         if (R > 8) return cudaErrorInvalidConfiguration;       // DSMEM variant needs a portable cluster
         return launch_clustered(search_kernel<Q, R, T, MINB>, a, rows, R, T, Smem<Q, R>::search, s);
@@ -1104,7 +1214,8 @@ struct Variant {
                           &launch_search_l2x, &max_clusters_l2x,
                           (size_t)2 * 16 * (Split<Q, R>::RS > GeoX<Q>::RSX ? Split<Q, R>::RS : GeoX<Q>::RSX) * sizeof(cf),
                           &launch_search_coop, &max_groups_coop,
-                          (size_t)R * SplitX<Q, R>::ACC_ELEMS * sizeof(float)};
+                          (size_t)R * SplitX<Q, R>::ACC_ELEMS * sizeof(float),
+                          &launch_wipe_pad, &launch_chirp_in, &launch_fine_chirp, &launch_chirp_out};
     }
 };
 

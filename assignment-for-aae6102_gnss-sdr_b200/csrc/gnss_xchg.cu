@@ -56,6 +56,7 @@ int xchg_begin(gnssacq_handle* h, const gnssacq_shard* sh, bool root, Xchg& x) {
     if (!h || !sh) return fail(h, GNSSACQ_ERR_INVALID_ARG, "NULL argument");
     if (h->xc.on) return fail(h, GNSSACQ_ERR_STATE, "exchange already set up on this handle");
     if (h->windows) return fail(h, GNSSACQ_ERR_STATE, "Doppler windows are set on this handle (clear them first)");
+    if (h->NF != h->N) return fail(h, GNSSACQ_ERR_STATE, "the multi-GPU exchange needs a built samples_per_ms (this handle zero-pads each ms)");
     if (sh->prn_count != h->P || sh->bin_count != h->B || sh->bin_first != h->bin0 || sh->freq_num_total != h->B_full ||
         (sh->plan_rows ? (sh->row_first != h->row0 || sh->row_count != h->n_rows) : (h->n_rows != h->P * h->B)))
         return fail(h, GNSSACQ_ERR_INVALID_ARG, "shard does not describe this handle (use gnssacq_shard_plan's config)");

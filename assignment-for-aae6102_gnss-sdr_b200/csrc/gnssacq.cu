@@ -349,10 +349,14 @@ const VariantOps* pick_variant(int Q, int R, int T) {
     return nullptr;
 }
 
-// Doppler bins -> (base transform, shift in FFT bins): f_b = f_base + s * (Fs/N)   (SURVEY A.7)
+// Doppler bins -> (base transform, shift in FFT bins): f_b = f_base + s * (Fs/NF)   (SURVEY A.7)
+// A padded shape (N < NF) with an M-ms fold also needs f_b - f_base to be a whole number of Fs/N: the carrier
+// advances by (f_b - f_base)*N/Fs cycles from one ms of the fold to the next, and only a whole number of cycles
+// leaves the folded block a plain shift of the base's (for N = NF both conditions are the same).
 void plan_bins(gnssacq_handle* h) {
     const gnssacq_config& c = h->cfg;
-    const double df = c.fs_hz / (double)c.samples_per_ms;
+    const double df = c.fs_hz / (double)h->NF, dms = c.fs_hz / (double)h->N;
+    const bool fold = h->M > 1 && h->NF != h->N;
     h->bin_base.assign(h->B, 0);
     h->bin_shift.assign(h->B, 0);
     h->base_freq.clear();
@@ -362,7 +366,9 @@ void plan_bins(gnssacq_handle* h) {
         for (size_t i = 0; i < h->base_freq.size(); ++i) {
             const double r = (f - h->base_freq[i]) / df;
             const double rr = std::nearbyint(r);
-            if (std::fabs(r - rr) * df < 1e-6 && std::fabs(rr) < (double)(c.samples_per_ms / 2)) {
+            const double q = (f - h->base_freq[i]) / dms;
+            if (std::fabs(r - rr) * df < 1e-6 && std::fabs(rr) < (double)(h->NF / 2) &&
+                (!fold || std::fabs(q - std::nearbyint(q)) * dms < 1e-6)) {
                 found = (int)i;
                 shift = (int)rr;
                 break;
@@ -389,6 +395,19 @@ int clear_unsearched(gnssacq_handle* h) {
     return GNSSACQ_OK;
 }
 
+// The transform length NF for N samples per ms: N itself when it is a built 2000*Q, otherwise the smallest built
+// length >= 2N - 1, into which each ms is zero-padded (the circular correlation of N lags then never wraps).
+// 0: neither (N > 29 000 and not built).
+int transform_length(int n) {
+    static const int kBuilt[] = {6000, 26000, 58000};         // 2000*Q, Q = 3, 13, 29 (gnss_q*.cu)
+    if (n <= 0) return 0;
+    for (int b : kBuilt)
+        if (n == b) return n;
+    for (int b : kBuilt)
+        if ((long long)b >= 2ll * n - 1) return b;
+    return 0;
+}
+
 int validate(const gnssacq_config* c, std::string& why) {
     if (!c) { why = "cfg is NULL"; return GNSSACQ_ERR_INVALID_ARG; }
     if (!(c->fs_hz > 0) || !(c->code_hz > 0)) { why = "fs_hz and code_hz must be positive"; return GNSSACQ_ERR_INVALID_ARG; }
@@ -409,8 +428,9 @@ int validate(const gnssacq_config* c, std::string& why) {
     }
     if (c->work_split < 0 || c->work_split > 2) { why = "work_split must be 0 (auto), 1 (whole rows) or 2 (block-granular tail)"; return GNSSACQ_ERR_INVALID_ARG; }
     if (c->exchange < 0 || c->exchange > 3) { why = "exchange must be 0 (auto), 1 (DSMEM), 2 (L2 + clusters) or 3 (L2 + cooperative groups)"; return GNSSACQ_ERR_INVALID_ARG; }
-    if (c->samples_per_ms <= 0 || c->samples_per_ms % 2000 != 0) {
-        why = "samples_per_ms must be 2000*Q (built: Q = 3, 13, 29 -> 6000, 26000, 58000)";
+    if (transform_length(c->samples_per_ms) == 0) {
+        why = "samples_per_ms must be a built transform length (6000, 26000, 58000) or at most 29000 "
+              "(zero-padded into the smallest built length >= 2*samples_per_ms - 1)";
         return GNSSACQ_ERR_UNSUPPORTED_N;
     }
     return GNSSACQ_OK;
@@ -521,11 +541,13 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
         wa.coh_ms = h->M;
         wa.K = h->K;
         wa.block_bytes = (size_t)h->N * h->M * h->cfg.data_type * h->cfg.data_precision;
+        wa.n_ms = h->N;
         wa.base_freq_hz = h->d_base_freq.get();
         wa.fs_hz = h->cfg.fs_hz;
         wa.means = means;
         wa.x = h->d_x.get();
-        CU(h->ops->launch_wipe(wa, (int)h->base_freq.size() * h->K, s));
+        if (h->NF == h->N) CU(h->ops->launch_wipe(wa, (int)h->base_freq.size() * h->K, s));
+        else CU(h->ops->launch_wipe_pad(wa, (int)h->base_freq.size() * h->K, s));
         h->launches += 1;
     }
     CU(cudaEventRecord(h->ev[2].get(), s));
@@ -538,6 +560,7 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
     sa.row_first = h->row0; sa.n_rows = h->n_rows;
     sa.rows = h->windows ? h->d_rows.get() : nullptr;
     sa.w = h->w;
+    sa.n_lags = h->N;
     sa.cand = xchg ? xc.cand_all + (size_t)xc.sh.prn_first * xc.sh.freq_num_total + xc.sh.bin_first : h->d_cand.get();
     sa.cand_stride = xchg ? xc.sh.freq_num_total : h->B;
     sa.surface = h->d_surface.get();
@@ -719,6 +742,14 @@ int gnssacq_code_replica(const gnssacq_config* c, int32_t prn, int8_t* out) {
     return GNSSACQ_OK;
 }
 
+int gnssacq_transform_size(const gnssacq_config* c, int32_t* n_out) {
+    if (!c || !n_out) return fail(nullptr, GNSSACQ_ERR_INVALID_ARG, "NULL argument");
+    const int nf = transform_length(c->samples_per_ms);
+    if (nf == 0) return fail(nullptr, GNSSACQ_ERR_UNSUPPORTED_N, "samples_per_ms has no built transform length (> 29 000 and not 6000, 26000 or 58000)");
+    *n_out = nf;
+    return GNSSACQ_OK;
+}
+
 const char* gnssacq_last_error(const gnssacq_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
 int gnssacq_destroy(gnssacq_handle* h) {
@@ -734,7 +765,8 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     int rc = validate(cfg, why);
     if (rc != GNSSACQ_OK) return fail(nullptr, rc, why);
 
-    const int Q = cfg->samples_per_ms / 2000;
+    const int NF = transform_length(cfg->samples_per_ms);       // validate() has checked it is not 0
+    const int Q = NF / 2000;
     const VariantOps* ops = pick_variant(Q, cfg->cluster_ctas, cfg->threads);
     if (!ops) {
         char buf[200];
@@ -767,6 +799,7 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     h->ops = ops;
     h->device = dev;
     h->N = cfg->samples_per_ms;
+    h->NF = NF;
     h->P = cfg->n_prn;
     h->B = cfg->freq_num;
     h->K = cfg->noncoh_blocks;
@@ -785,7 +818,7 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     }
     h->row0 = cfg->row_count > 0 ? cfg->row_first : 0;
     h->n_rows = cfg->row_count > 0 ? cfg->row_count : h->P * h->B;
-    const size_t N = (size_t)h->N;
+    const size_t N = (size_t)h->N, NFs = (size_t)NF;
     const size_t nb = h->base_freq.size();
 
     CU(cudaSetDevice(dev), GNSSACQ_ERR_NOMEM);
@@ -794,9 +827,9 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     for (auto& e : h->ev) CU(create(e, cudaEventDefault), GNSSACQ_ERR_NOMEM);
     CU(ops->prepare(), GNSSACQ_ERR_NOMEM);
     CU(alloc(h->d_if, h->if_bytes), GNSSACQ_ERR_NOMEM);
-    CU(alloc(h->d_scode, (size_t)h->P * N), GNSSACQ_ERR_NOMEM);
-    CU(alloc(h->d_cc, (size_t)h->P * N * sizeof(cf)), GNSSACQ_ERR_NOMEM);
-    CU(alloc(h->d_x, nb * (size_t)h->K * (N / (N / 2000) * (2 * (N / 2000) - 1)) * sizeof(cf)), GNSSACQ_ERR_NOMEM);   // c-extended: N*(2Q-1)/Q
+    CU(alloc(h->d_scode, (size_t)h->P * NFs), GNSSACQ_ERR_NOMEM);
+    CU(alloc(h->d_cc, (size_t)h->P * NFs * sizeof(cf)), GNSSACQ_ERR_NOMEM);
+    CU(alloc(h->d_x, nb * (size_t)h->K * (NFs / Q * (2 * Q - 1)) * sizeof(cf)), GNSSACQ_ERR_NOMEM);   // c-extended: NF*(2Q-1)/Q
     CU(alloc(h->d_bin_base, h->B * sizeof(int)), GNSSACQ_ERR_NOMEM);
     CU(alloc(h->d_bin_shift, h->B * sizeof(int)), GNSSACQ_ERR_NOMEM);
     CU(alloc(h->d_prn, h->P * sizeof(int)), GNSSACQ_ERR_NOMEM);
@@ -831,10 +864,11 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
     }
     std::vector<double> bw(nb);                                 // (read by a copy that the final sync waits for)
     {
-        // K1 v2 (comb rows + cp.async staging) whenever its shared memory fits; otherwise the v1 gather kernel
+        // K1 v2 (comb rows + cp.async staging) whenever its shared memory fits; otherwise, and for every padded shape
+        // (its ms are not whole comb rows), the v1 gather kernel
         const int bps = h->cfg.data_type * h->cfg.data_precision;
         const int pitch = ((N / 16) * bps + 15) / 16 * 16;
-        if (ops->smem_wipe2(pitch, h->M) <= (size_t)227 * 1024) {
+        if (NF == h->N && ops->smem_wipe2(pitch, h->M) <= (size_t)227 * 1024) {
             for (size_t i = 0; i < nb; ++i) bw[i] = h->base_freq[i] / h->cfg.fs_hz;
             CU(alloc(h->d_base_w, nb * sizeof(double)), GNSSACQ_ERR_NOMEM);
             CU(cudaMemcpyAsync(h->d_base_w.get(), bw.data(), nb * sizeof(double), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
@@ -845,15 +879,43 @@ int gnssacq_create(const gnssacq_config* cfg, gnssacq_handle** out) {
         }
     }
 
-    // code tables -> HBM, then K0 fills the conj-spectrum cache
+    // code tables -> HBM, then K0 fills the conj-spectrum cache with conj(fft(c2))/NF: c2[j] = c[j mod N] for
+    // j <= 2N-2, 0 beyond (c2 = c for N = NF), so that lags m < N of the NF-point correlation never wrap
+    std::vector<cf> chirp, hfilt;                                // (padded: read by copies that the final sync waits for)
     {
-        std::vector<int8_t> sc((size_t)h->P * N);
-        for (int p = 0; p < h->P; ++p) code_replica(*cfg, cfg->prn[p], sc.data() + (size_t)p * N);
+        std::vector<int8_t> sc((size_t)h->P * NFs, 0), one(N);
+        for (int p = 0; p < h->P; ++p) {
+            code_replica(*cfg, cfg->prn[p], one.data());
+            int8_t* row = sc.data() + (size_t)p * NFs;
+            for (size_t j = 0; j < NFs && j <= 2 * N - 2; ++j) row[j] = one[j % N];
+        }
         CU(cudaMemcpyAsync(h->d_scode.get(), sc.data(), sc.size(), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
         CodeArgs a{h->d_scode.get(), h->d_cc.get()};
         CU(ops->launch_code(a, h->P, h->stream), GNSSACQ_ERR_NOMEM);
-        CU(cudaStreamSynchronize(h->stream), GNSSACQ_ERR_NOMEM);
     }
+    if (NF != h->N) {
+        // Bluestein tables of the N-point DFTs (fine stage, gnssacq_fft_forward): ch[n] = exp(i pi n^2 / N) with n^2 mod 2N
+        // in integers (exact: 2N^2 < 2^31 for N <= 29 000), and H = FFT_NF of the chirp filter h[j] = ch[|j|], |j| < N
+        chirp.resize(N);
+        hfilt.assign(NFs, mk(0.f, 0.f));
+        for (int n = 0; n < h->N; ++n) {
+            const int e = (int)(((long long)n * n) % (2ll * h->N));
+            const double ang = 3.14159265358979323846 * (double)e / (double)h->N;
+            chirp[n] = mk((float)std::cos(ang), (float)std::sin(ang));
+            hfilt[n] = chirp[n];
+            if (n > 0) hfilt[NFs - n] = chirp[n];
+        }
+        CU(alloc(h->d_chirp, N * sizeof(cf)), GNSSACQ_ERR_NOMEM);
+        CU(alloc(h->d_chirp_filt, NFs * sizeof(cf)), GNSSACQ_ERR_NOMEM);
+        DevPtr<cf> tmp;
+        CU(alloc(tmp, NFs * sizeof(cf)), GNSSACQ_ERR_NOMEM);
+        CU(cudaMemcpyAsync(h->d_chirp.get(), chirp.data(), N * sizeof(cf), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
+        CU(cudaMemcpyAsync(tmp.get(), hfilt.data(), NFs * sizeof(cf), cudaMemcpyHostToDevice, h->stream), GNSSACQ_ERR_NOMEM);
+        NaturalArgs na{tmp.get(), h->d_chirp_filt.get()};
+        CU(ops->launch_natural(na, 1, h->stream), GNSSACQ_ERR_NOMEM);
+        CU(cudaStreamSynchronize(h->stream), GNSSACQ_ERR_NOMEM);   // before `tmp` is freed
+    }
+    CU(cudaStreamSynchronize(h->stream), GNSSACQ_ERR_NOMEM);
     *out = owner.release();
     return GNSSACQ_OK;
 }
@@ -1032,7 +1094,9 @@ int gnssacq_fine_frequency(gnssacq_handle* h, const void* if_long, size_t nbytes
     const long long LN = (long long)L * N, F = LN * K;                          // acquisition.m:108
     if (F > 0xFFFFFFFFll) return fail(h, GNSSACQ_ERR_INVALID_ARG, "fftlength exceeds 2^32");
 
-    constexpr int kChunk = 4;                                                   // SVs per pass (scratch ~0.4 GB at N = 58 000)
+    constexpr int kChunk = 4;                                                   // SVs per pass (scratch ~0.4 GB at N = 58 000;
+                                                                                // a padded shape adds K*L*NF per SV: ~0.37 GB at 16.368 MHz, L = 10, K = 20)
+    const bool padded = h->NF != h->N;
     if (!h->fine || h->fine->L != L) {
         // (re)build the per-L scratch: chip index of sample t (acquisition.m:104-105, same double arithmetic)
         h->fine.reset();                                                        // the old scratch goes first
@@ -1050,6 +1114,7 @@ int gnssacq_fine_frequency(gnssacq_handle* h, const void* if_long, size_t nbytes
         CU(alloc(fs->start, GNSSACQ_MAX_PRN * sizeof(int)));
         CU(alloc(fs->best, GNSSACQ_MAX_PRN * sizeof(unsigned long long)));
         CU(alloc(fs->u, (size_t)kChunk * K * L * N * sizeof(cf)));
+        if (padded) CU(alloc(fs->v, (size_t)kChunk * K * L * h->NF * sizeof(cf)));
         CU(cudaMemcpyAsync(fs->chip.get(), chip.data(), chip.size() * sizeof(uint16_t), cudaMemcpyHostToDevice, s));
         CU(cudaStreamSynchronize(s));                                           // `chip` is a temporary
         fs->L = L;
@@ -1083,7 +1148,14 @@ int gnssacq_fine_frequency(gnssacq_handle* h, const void* if_long, size_t nbytes
         fa.raw = d_raw; fa.chip = d_chip; fa.ca = d_ca + (size_t)first * 1023; fa.start = d_start + first;
         fa.means = means; fa.data_type = c.data_type; fa.precision = c.data_precision;
         fa.L = L; fa.K = K; fa.F = F; fa.u = d_u;
-        CU(h->ops->launch_fine(fa, n * K * L, s));
+        if (padded) {
+            // the K*L N-point DFTs as Bluestein convolutions through the NF-point engine (see ChirpArgs)
+            ChirpArgs ca{h->d_chirp.get(), h->d_chirp_filt.get(), N, nullptr, h->fine->v.get(), d_u};
+            CU(h->ops->launch_fine_chirp(fa, ca, n * K * L, s));
+            CU(h->ops->launch_chirp_out(ca, n * K * L, s));
+        } else {
+            CU(h->ops->launch_fine(fa, n * K * L, s));
+        }
         dim3 grid((unsigned)((N + 255) / 256), (unsigned)K, (unsigned)n);
         fine_combine_kernel<<<grid, 256, 0, s>>>(d_u, K, L, N, F, c.data_type == 2 ? 1 : 0, d_best + first);
         CU(cudaGetLastError());
@@ -1134,15 +1206,24 @@ int gnssacq_fft_forward(gnssacq_handle* h, const float* in, float* out) {
     if (!h || !in || !out) return fail(h, GNSSACQ_ERR_INVALID_ARG, "NULL argument");
     CU(cudaSetDevice(h->device));
     const size_t bytes = (size_t)h->N * sizeof(cf);
+    const bool padded = h->NF != h->N;
     if (!h->fft) {
         auto f = std::make_unique<FftState>();
         CU(alloc(f->in, bytes));
         CU(alloc(f->out, bytes));
+        if (padded) CU(alloc(f->v, (size_t)h->NF * sizeof(cf)));
         h->fft = std::move(f);
     }
     CU(cudaMemcpyAsync(h->fft->in.get(), in, bytes, cudaMemcpyHostToDevice, h->stream));
-    NaturalArgs a{h->fft->in.get(), h->fft->out.get()};
-    CU(h->ops->launch_natural(a, 1, h->stream));
+    if (padded) {
+        // the N-point DFT as a Bluestein convolution through the NF-point engine (the fine stage's path)
+        ChirpArgs c{h->d_chirp.get(), h->d_chirp_filt.get(), h->N, h->fft->in.get(), h->fft->v.get(), h->fft->out.get()};
+        CU(h->ops->launch_chirp_in(c, 1, h->stream));
+        CU(h->ops->launch_chirp_out(c, 1, h->stream));
+    } else {
+        NaturalArgs a{h->fft->in.get(), h->fft->out.get()};
+        CU(h->ops->launch_natural(a, 1, h->stream));
+    }
     CU(cudaMemcpyAsync(out, h->fft->out.get(), bytes, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     return GNSSACQ_OK;

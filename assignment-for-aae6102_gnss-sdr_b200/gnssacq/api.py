@@ -118,7 +118,7 @@ EXPORTS = (
     "gnssacq_loop_params_default", "gnssacq_track",
     "gnssacq_shard_plan", "gnssacq_shard_plan_rows", "gnssacq_xchg_root", "gnssacq_xchg_attach", "gnssacq_xchg_attach_local",
     "gnssacq_xchg_if_buffer", "gnssacq_xchg_enqueue", "gnssacq_xchg_finish", "gnssacq_xchg_fetch",
-    "gnssacq_set_doppler_windows",
+    "gnssacq_set_doppler_windows", "gnssacq_transform_size",
 )
 
 
@@ -167,6 +167,7 @@ def _load() -> C.CDLL:
     lib.gnssacq_xchg_fetch.argtypes = [vp, C.POINTER(Result), C.POINTER(Stats)]
     lib.gnssacq_fp32_peak_tflops.argtypes = [C.c_int32, C.POINTER(C.c_double)]
     lib.gnssacq_set_doppler_windows.argtypes = [vp, vp, vp]
+    lib.gnssacq_transform_size.argtypes = [C.POINTER(Config), C.POINTER(C.c_int32)]
     return lib
 
 
@@ -249,6 +250,16 @@ def code_replica(cfg: Config, prn: int) -> np.ndarray:
     if rc:
         raise GnssAcqError(rc, STATUS.get(rc, "?"))
     return out
+
+
+def transform_size(cfg: Config) -> int:
+    """Transform length a search of ``cfg.samples_per_ms`` runs on (gnssacq_transform_size): samples_per_ms itself
+    when it is built (6000, 26000, 58000), else the built length each ms is zero-padded into.  No device needed."""
+    n = C.c_int32()
+    rc = lib.gnssacq_transform_size(C.byref(cfg), C.byref(n))
+    if rc:
+        raise GnssAcqError(rc, (lib.gnssacq_last_error(None) or b"").decode())
+    return n.value
 
 
 def search_multi(searchers: Sequence["Searcher"], if_bytes) -> List[Result]:

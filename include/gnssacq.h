@@ -30,7 +30,8 @@ extern "C" {
 typedef enum gnssacq_status {
     GNSSACQ_OK = 0,
     GNSSACQ_ERR_INVALID_ARG = -1,    /* NULL pointer, non-positive count, PRN outside 1..51 ...        */
-    GNSSACQ_ERR_UNSUPPORTED_N = -2,  /* samples_per_ms is not 2000*Q with Q in the built set           */
+    GNSSACQ_ERR_UNSUPPORTED_N = -2,  /* samples_per_ms has no transform length: neither 2000*Q with Q
+                                        built (6000, 26000, 58000) nor <= 29000 (gnssacq_transform_size) */
     GNSSACQ_ERR_SHORT_BUFFER = -3,   /* fewer IF bytes than noncoh_blocks*coh_ms ms                    */
     GNSSACQ_ERR_CUDA = -4,           /* a CUDA runtime call failed; see gnssacq_last_error             */
     GNSSACQ_ERR_NO_DEVICE = -5,      /* no CUDA device / wrong architecture                            */
@@ -44,7 +45,9 @@ typedef struct gnssacq_config {
     double fs_hz;             /* signal.Fs            (initParameters.m:42) */
     double if_hz;             /* signal.IF            (initParameters.m:41) */
     double code_hz;           /* signal.codeFreqBasis (initParameters.m:44) */
-    int32_t samples_per_ms;   /* signal.Sample = ceil(Fs*1e-3) (initParameters.m:46) */
+    int32_t samples_per_ms;   /* signal.Sample = ceil(Fs*1e-3) (initParameters.m:46).  Any value up to 29000
+                                 (Fs <= 29 MHz), or 58000: a value that is not a built transform length is
+                                 zero-padded each ms into one (gnssacq_transform_size) */
     int32_t data_type;        /* file.dataType: 1 real, 2 I/Q   (initParameters.m:37) */
     int32_t data_precision;   /* file.dataPrecision: 1 int8, 2 int16 (initParameters.m:38) */
     double freq_min_hz;       /* acq.freqMin  (initParameters.m:52) */
@@ -125,6 +128,13 @@ int gnssacq_config_default(gnssacq_config* cfg);
 /* Bytes of IF data one search consumes: samples_per_ms*data_type*data_precision*noncoh_blocks*coh_ms
  * (the fread count of acquisition.m:29/34 times the sample size). */
 size_t gnssacq_if_bytes(const gnssacq_config* cfg);
+
+/* Transform length the search of cfg->samples_per_ms = N runs on: N itself when N is a built 2000*Q (6000,
+ * 26000, 58000), otherwise the smallest built length >= 2N-1, into which each ms is zero-padded (the same rows
+ * as a circular N-point correlation, at the cost of the longer transform).  Host only, no device needed.
+ * Returns GNSSACQ_ERR_UNSUPPORTED_N, as gnssacq_create does, when there is none (N > 29000, not built).
+ * A handle whose N is padded cannot take part in the multi-GPU exchange (gnssacq_xchg_*: GNSSACQ_ERR_STATE). */
+int gnssacq_transform_size(const gnssacq_config* cfg, int32_t* n_out);
 
 /* Build a handle: validates cfg, selects the device, allocates HBM/pinned buffers and fills the
  * HBM-resident cache of conj(fft(code))/N for cfg->prn[] (replaces acquisition.m:49-51,58). */
@@ -320,7 +330,9 @@ int gnssacq_read_surface(gnssacq_handle* h, int32_t prn_index, float* out);
  * loop on every SM, CUDA-event timed): the denominator of the FP32 roofline, since
  * MEASURED_PEAKS.json only records HBM and BF16 tensor peaks. */
 int gnssacq_fp32_peak_tflops(int32_t device, double* out_tflops);
-/* Forward DFT of samples_per_ms complex floats (interleaved re,im; host pointers) through the engine. */
+/* Forward DFT of samples_per_ms complex floats (interleaved re,im; host pointers) through the engine.  For a
+ * padded samples_per_ms N the N-point DFT is a Bluestein (chirp-z) convolution through the engine's longer
+ * transform, the same path as the fine-frequency stage's DFTs. */
 int gnssacq_fft_forward(gnssacq_handle* h, const float* in, float* out);
 
 #ifdef __cplusplus
