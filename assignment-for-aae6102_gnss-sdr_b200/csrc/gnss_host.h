@@ -175,6 +175,8 @@ struct gnssacq_handle {
     std::unique_ptr<gnss::TrackState> trk;
     gnss::DevPtr<gnssacq_track_record> d_trk_rec;   // [channels][periods]
     size_t trk_rec_cap = 0;
+    gnss::DevPtr<double> d_trk_bank;       // gnssacq_track_bank: [I, Q][channels][periods][taps], trk_bank_cap per plane
+    size_t trk_bank_cap = 0;
     // pinned host
     gnss::PinnedPtr<void> h_if;
     gnss::PinnedPtr<gnssacq_result> h_res;

@@ -1,6 +1,7 @@
 // gnss_track.cu -- tracking on the resident recording (include/gnssacq.h: gnssacq_track_load, gnssacq_correlate,
-// gnssacq_track): K7 correlators for a batch of channels, K8 the whole DLL/PLL loop on the device.
+// gnssacq_track, gnssacq_track_bank): K7 correlators for a batch of channels, K8 the whole DLL/PLL loop on the device.
 #include <cooperative_groups.h>
+#include <cmath>
 #include <vector>
 
 #include "gnss_host.h"
@@ -141,10 +142,77 @@ struct LoopArgs {
     int n_periods;
     gnssacq_track_record* out;
     int* status;              // != 0: some channel ran out of samples
+    // gnssacq_track_bank only (track_loop_kernel<true>): the bank observed every period
+    int n_taps;
+    const double* spacing;    // [n_taps]
+    double* bank_i;           // [channels][n_periods][n_taps]
+    double* bank_q;
 };
 
 __device__ __forceinline__ double round_half_away(double v) { return v < 0.0 ? -floor(-v + 0.5) : floor(v + 0.5); }
 
+// The bank's per-CTA staging: per-warp sums, the double-buffered slots that the period's cluster barrier publishes
+// together with slot[par], the taps' spacings and the channel's chips.  [iq * kTrackMaxTaps + tap]
+struct BankSmem {
+    double wsum[kLoopThreads / 32][2 * kTrackMaxTaps];
+    double slot[2][2 * kTrackMaxTaps];
+    double spacing[kTrackMaxTaps];
+    int8_t ca[1024];
+};
+__device__ __forceinline__ BankSmem& bank_smem() { __shared__ BankSmem s; return s; }   // track_loop_kernel<true> only
+
+// Taps tap0 .. tap0+G-1 of the bank over this thread's samples of the period (n = gtid + j*gthreads), with the E/P/L
+// loop's sample conversion, carrier rotation from (sn, cs) and code-index rule; lane 0 leaves the warp's sums in
+// bs.wsum.  (__double2int_ru is (int)ceil in one conversion, and the chip is +-1, so adding +-inph is chip * inph:
+// the same doubles as the E/P/L taps.)
+template <int G>
+__device__ __forceinline__ void bank_taps(const LoopArgs& a, BankSmem& bs, int tap0, int gtid, int gthreads, long long pos,
+                                          int ns, double rem_chip, double step, double mi, double mq, double sn, double cs,
+                                          double rc, double rs) {
+    double off[G], acc_i[G], acc_q[G];
+#pragma unroll
+    for (int t = 0; t < G; ++t) {
+        off[t] = (0.0 + bs.spacing[tap0 + t]) + rem_chip;
+        acc_i[t] = acc_q[t] = 0.0;
+    }
+    for (int n = gtid; n < ns; n += gthreads) {
+        const long long idx = pos + n;
+        float fr, fi = 0.f;
+        if (a.precision == 2) { const short2 v = ((const short2*)a.raw)[idx]; fr = (float)v.x; fi = (float)v.y; }
+        else if (a.data_type == 2) { const char2 v = ((const char2*)a.raw)[idx]; fr = (float)v.x; fi = (float)v.y; }
+        else fr = (float)((const int8_t*)a.raw)[idx];
+        const double xr = (double)fr - mi, xi = (a.data_type == 2 || a.precision == 2) ? (double)fi - mq : 0.0;
+        const double inph = xr * sn + xi * cs, quad = xr * cs - xi * sn;
+        const double cn = cs * rc - sn * rs;
+        sn = sn * rc + cs * rs;
+        cs = cn;
+        const double sn_d = __dmul_rn(step, (double)n);
+#pragma unroll
+        for (int t = 0; t < G; ++t) {
+            int k = __double2int_ru(__dadd_rn(off[t], sn_d)) - 1;
+            k %= 1023;
+            if (k < 0) k += 1023;
+            const bool neg = bs.ca[k] < 0;
+            acc_i[t] += neg ? -inph : inph;
+            acc_q[t] += neg ? -quad : quad;
+        }
+    }
+#pragma unroll
+    for (int t = 0; t < G; ++t) {
+        for (int o = 16; o; o >>= 1) {
+            acc_i[t] += __shfl_down_sync(0xffffffffu, acc_i[t], o);
+            acc_q[t] += __shfl_down_sync(0xffffffffu, acc_q[t], o);
+        }
+        if ((threadIdx.x & 31) == 0) {
+            bs.wsum[threadIdx.x >> 5][tap0 + t] = acc_i[t];
+            bs.wsum[threadIdx.x >> 5][kTrackMaxTaps + tap0 + t] = acc_q[t];
+        }
+    }
+}
+
+// kBank = false: gnssacq_track.  kBank = true: gnssacq_track_bank, the same loop observed by n_taps more taps,
+// summed after the E/P/L taps and published by the same cluster barrier; nothing of the loop reads them.
+template <bool kBank>
 __global__ void __launch_bounds__(kLoopThreads, 1) track_loop_kernel(LoopArgs a) {
     namespace cgx = cooperative_groups;
     cgx::cluster_group cluster = cgx::this_cluster();
@@ -175,6 +243,11 @@ __global__ void __launch_bounds__(kLoopThreads, 1) track_loop_kernel(LoopArgs a)
         st.ns = (int)round_half_away((1023.0 - rem_chip) / st.step);                  // :78 (pdi = 1)
         st.stop = (st.ns < 1 || pos + st.ns > a.total_samples) ? 1 : 0;               // :107-111
     };
+    if constexpr (kBank) {
+        BankSmem& bs = bank_smem();
+        for (int k = threadIdx.x; k < 1023; k += kLoopThreads) bs.ca[k] = ca[k];
+        if (threadIdx.x < a.n_taps) bs.spacing[threadIdx.x] = a.spacing[threadIdx.x];
+    }
     if (threadIdx.x == 0) publish(state[0], c0.rem_chip, c0.rem_phase, c0.code_hz, c0.carrier_hz, c0.sample_offset);
     __syncthreads();
 
@@ -260,11 +333,31 @@ __global__ void __launch_bounds__(kLoopThreads, 1) track_loop_kernel(LoopArgs a)
             for (int o = 16; o; o >>= 1) acc[t] += __shfl_down_sync(0xffffffffu, acc[t], o);
             if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5][t] = acc[t];
         }
+        if constexpr (kBank) {                 // second pass over the thread's samples (just read: L1/L2-resident)
+            BankSmem& bs = bank_smem();
+            double cs0, sn0, rc0, rs0;         // the E/P/L loop's start phasor and rotation, recomputed
+            sincos(__dadd_rn(__dmul_rn(two_pi, __dmul_rn(carrier_hz, (double)gtid / a.fs_hz)), rem_phase), &sn0, &cs0);
+            sincos(two_pi * (carrier_hz * ((double)gthreads / a.fs_hz)), &rs0, &rc0);
+            int t0 = 0;
+            for (; t0 + 8 <= a.n_taps; t0 += 8) bank_taps<8>(a, bs, t0, gtid, gthreads, pos, ns, rem_chip, step, mi, mq, sn0, cs0, rc0, rs0);
+            if (a.n_taps - t0 >= 4) { bank_taps<4>(a, bs, t0, gtid, gthreads, pos, ns, rem_chip, step, mi, mq, sn0, cs0, rc0, rs0); t0 += 4; }
+            if (a.n_taps - t0 >= 2) { bank_taps<2>(a, bs, t0, gtid, gthreads, pos, ns, rem_chip, step, mi, mq, sn0, cs0, rc0, rs0); t0 += 2; }
+            if (a.n_taps - t0 >= 1) bank_taps<1>(a, bs, t0, gtid, gthreads, pos, ns, rem_chip, step, mi, mq, sn0, cs0, rc0, rs0);
+        }
         __syncthreads();
         if (threadIdx.x < 6) {
             double v = 0.0;
             for (int w = 0; w < kLoopThreads / 32; ++w) v += wsum[w][threadIdx.x];
             slot[par][threadIdx.x] = v;
+        }
+        if constexpr (kBank) {                 // warps 2-3: the CTA's bank sums, beside slot[par]
+            BankSmem& bs = bank_smem();
+            const int j = (int)threadIdx.x - 64;
+            if (j >= 0 && j < 2 * kTrackMaxTaps && (j & (kTrackMaxTaps - 1)) < a.n_taps) {
+                double v = 0.0;
+                for (int w = 0; w < kLoopThreads / 32; ++w) v += bs.wsum[w][j];
+                bs.slot[par][j] = v;
+            }
         }
         cluster.sync();                                                               // release/acquire: all slots visible
         if (threadIdx.x < 6) {                                                        // six threads pull the eight slots
@@ -296,6 +389,15 @@ __global__ void __launch_bounds__(kLoopThreads, 1) track_loop_kernel(LoopArgs a)
                 r.rem_chip = n_rem_chip; r.code_hz = n_code_hz; r.carrier_hz = n_carrier_hz; r.rem_phase = n_rem_phase;
                 r.sample_end = pos + ns; r.num_samples = ns; r.reserved = 0;
                 a.out[(size_t)cidx * a.n_periods + period] = r;
+            }
+        }
+        if constexpr (kBank) {                             // rank 0's warps 2-3 store the bank while thread 0 runs the loop
+            BankSmem& bs = bank_smem();                    // math; the slots are rewritten two cluster barriers from now
+            const int j = (int)threadIdx.x - 64, t = j & (kTrackMaxTaps - 1);
+            if (rank == 0 && j >= 0 && j < 2 * kTrackMaxTaps && t < a.n_taps) {
+                double v = 0.0;
+                for (int r = 0; r < kLoopCtas; ++r) v += cluster.map_shared_rank(&bs.slot[par][0], r)[j];
+                (j < kTrackMaxTaps ? a.bank_i : a.bank_q)[((size_t)cidx * a.n_periods + period) * a.n_taps + t] = v;
             }
         }
         __syncthreads();                                   // state[par ^ 1] is complete
@@ -394,8 +496,12 @@ int gnssacq_loop_params_default(gnssacq_loop_params* p) {
     return GNSSACQ_OK;
 }
 
-int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start, const gnssacq_loop_params* loops,
-                  int32_t n_periods, gnssacq_track_record* out) {
+}  // extern "C"
+
+// gnssacq_track (n_taps == 0) and gnssacq_track_bank (bank arguments already checked)
+static int track_run(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start, const gnssacq_loop_params* loops,
+                     int32_t n_periods, gnssacq_track_record* out, int32_t n_taps, const double* spacing_chips,
+                     double* bank_i, double* bank_q) {
     if (!h || !start || !loops || !out) return fail(h, GNSSACQ_ERR_INVALID_ARG, "NULL argument");
     if (!h->d_trk_raw || !h->trk_bytes) return fail(h, GNSSACQ_ERR_STATE, "gnssacq_track_load first");
     if (n_channels < 1 || n_channels > kTrackMaxChannels || n_periods < 1)
@@ -420,8 +526,19 @@ int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* 
         CU(alloc(h->d_trk_rec, n_rec * sizeof(gnssacq_track_record)));
         h->trk_rec_cap = n_rec;
     }
+    const size_t n_bank = n_rec * (size_t)n_taps;                    // per plane
+    if (h->trk_bank_cap < n_bank) {                                  // 64 channels x 1e5 periods x 32 taps: 3.3 GB
+        CU(cudaStreamSynchronize(s));
+        h->trk_bank_cap = 0;
+        CU(alloc(h->d_trk_bank, 2 * n_bank * sizeof(double)), GNSSACQ_ERR_NOMEM);
+        h->trk_bank_cap = n_bank;
+    }
     CU(cudaMemsetAsync(h->trk->status.get(), 0, sizeof(int), s));
     CU(cudaMemsetAsync(h->d_trk_rec.get(), 0, n_rec * sizeof(gnssacq_track_record), s));
+    if (n_taps) {
+        CU(cudaMemsetAsync(h->d_trk_bank.get(), 0, 2 * n_bank * sizeof(double), s));
+        CU(cudaMemcpyAsync(h->trk->spacing.get(), spacing_chips, n_taps * sizeof(double), cudaMemcpyHostToDevice, s));
+    }
     CU(cudaMemcpyAsync(h->trk->ch.get(), start, n_channels * sizeof(gnssacq_channel), cudaMemcpyHostToDevice, s));
     LoopArgs a;
     a.raw = h->d_trk_raw.get();
@@ -436,6 +553,10 @@ int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* 
     a.n_periods = n_periods;
     a.out = h->d_trk_rec.get();
     a.status = h->trk->status.get();
+    a.n_taps = n_taps;
+    a.spacing = h->trk->spacing.get();
+    a.bank_i = h->d_trk_bank.get();
+    a.bank_q = a.bank_i ? a.bank_i + n_bank : nullptr;
     cudaLaunchConfig_t lc = {};
     lc.gridDim = dim3((unsigned)(n_channels * kLoopCtas), 1, 1);
     lc.blockDim = dim3(kLoopThreads, 1, 1);
@@ -448,13 +569,35 @@ int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* 
     attr[0].val.clusterDim.z = 1;
     lc.attrs = attr;
     lc.numAttrs = 1;
-    CU(cudaLaunchKernelEx(&lc, track_loop_kernel, a));
+    if (n_taps) CU(cudaLaunchKernelEx(&lc, track_loop_kernel<true>, a));
+    else CU(cudaLaunchKernelEx(&lc, track_loop_kernel<false>, a));
     int status = 0;
     CU(cudaMemcpyAsync(out, h->d_trk_rec.get(), n_rec * sizeof(gnssacq_track_record), cudaMemcpyDeviceToHost, s));
+    if (n_taps) {
+        CU(cudaMemcpyAsync(bank_i, a.bank_i, n_bank * sizeof(double), cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(bank_q, a.bank_q, n_bank * sizeof(double), cudaMemcpyDeviceToHost, s));
+    }
     CU(cudaMemcpyAsync(&status, h->trk->status.get(), sizeof(int), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     if (status) return fail(h, GNSSACQ_ERR_SHORT_BUFFER, "Not enough raw data (trackingCT.m:107-111): a channel ran past the loaded segment");
     return GNSSACQ_OK;
+}
+
+extern "C" {
+
+int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start, const gnssacq_loop_params* loops,
+                  int32_t n_periods, gnssacq_track_record* out) {
+    return track_run(h, n_channels, start, loops, n_periods, out, 0, nullptr, nullptr, nullptr);
+}
+
+int gnssacq_track_bank(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start,
+                       const gnssacq_loop_params* loops, int32_t n_periods, int32_t n_taps, const double* spacing_chips,
+                       gnssacq_track_record* out, double* bank_i, double* bank_q) {
+    if (!spacing_chips || !bank_i || !bank_q) return fail(h, GNSSACQ_ERR_INVALID_ARG, "NULL argument");
+    if (n_taps < 1 || n_taps > kTrackMaxTaps) return fail(h, GNSSACQ_ERR_INVALID_ARG, "1..32 taps");
+    for (int t = 0; t < n_taps; ++t)
+        if (!std::isfinite(spacing_chips[t])) return fail(h, GNSSACQ_ERR_INVALID_ARG, "spacing must be finite");
+    return track_run(h, n_channels, start, loops, n_periods, out, n_taps, spacing_chips, bank_i, bank_q);
 }
 
 }  // extern "C"

@@ -115,7 +115,7 @@ EXPORTS = (
     "gnssacq_search_device", "gnssacq_enqueue_device", "gnssacq_enqueue_device_out", "gnssacq_fetch_results",
     "gnssacq_ca_code", "gnssacq_code_replica", "gnssacq_read_surface", "gnssacq_fft_forward", "gnssacq_fp32_peak_tflops", "gnssacq_fine_frequency",
     "gnssacq_search_multi", "gnssacq_sweep", "gnssacq_sweep_file", "gnssacq_track_load", "gnssacq_correlate",
-    "gnssacq_loop_params_default", "gnssacq_track",
+    "gnssacq_loop_params_default", "gnssacq_track", "gnssacq_track_bank",
     "gnssacq_shard_plan", "gnssacq_shard_plan_rows", "gnssacq_xchg_root", "gnssacq_xchg_attach", "gnssacq_xchg_attach_local",
     "gnssacq_xchg_if_buffer", "gnssacq_xchg_enqueue", "gnssacq_xchg_finish", "gnssacq_xchg_fetch",
     "gnssacq_set_doppler_windows", "gnssacq_transform_size",
@@ -152,6 +152,8 @@ def _load() -> C.CDLL:
     lib.gnssacq_track_load.argtypes = [vp, vp, C.c_size_t]
     lib.gnssacq_loop_params_default.argtypes = [C.POINTER(LoopParams)]
     lib.gnssacq_track.argtypes = [vp, C.c_int32, C.POINTER(Channel), C.POINTER(LoopParams), C.c_int32, C.POINTER(TrackRecord)]
+    lib.gnssacq_track_bank.argtypes = [vp, C.c_int32, C.POINTER(Channel), C.POINTER(LoopParams), C.c_int32, C.c_int32, vp,
+                                       C.POINTER(TrackRecord), vp, vp]
     lib.gnssacq_correlate.argtypes = [vp, C.c_int32, C.POINTER(Channel), C.c_int32, vp, vp, vp]
     lib.gnssacq_sweep.argtypes = [vp, C.POINTER(vp), C.c_int32, C.c_size_t, C.POINTER(Result), C.POINTER(Stats)]
     lib.gnssacq_sweep_file.argtypes = [vp, C.c_char_p, C.c_int64, C.c_int32, C.c_int32, C.POINTER(Result), C.POINTER(Stats)]
@@ -443,6 +445,23 @@ class Searcher:
         out = (TrackRecord * (n * n_periods))()
         self._check(lib.gnssacq_track(self._h, n, ch, C.byref(loops), n_periods, out))
         return [list(out[i * n_periods:(i + 1) * n_periods]) for i in range(n)]
+
+    def track_bank(self, start: Sequence["Channel"], n_periods: int, spacing_chips: Sequence[float],
+                   loops: Optional["LoopParams"] = None):
+        """`track`, and every period the correlator bank at `spacing_chips` (it only observes the loop): (records,
+        bank_i, bank_q), records as `track` returns them, bank_i / bank_q float64 [n_channels, n_periods, n_taps]."""
+        if loops is None:
+            loops = LoopParams()
+            lib.gnssacq_loop_params_default(C.byref(loops))
+        n = len(start)
+        ch = (Channel * n)(*start)
+        sp = np.ascontiguousarray(spacing_chips, dtype=np.float64)
+        out = (TrackRecord * (n * n_periods))()
+        bank_i = np.zeros((n, n_periods, sp.size), dtype=np.float64)
+        bank_q = np.zeros((n, n_periods, sp.size), dtype=np.float64)
+        self._check(lib.gnssacq_track_bank(self._h, n, ch, C.byref(loops), n_periods, sp.size, sp.ctypes.data, out,
+                                           bank_i.ctypes.data, bank_q.ctypes.data))
+        return [list(out[i * n_periods:(i + 1) * n_periods]) for i in range(n)], bank_i, bank_q
 
     def search_device(self, dev_ptr: int, nbytes: int) -> List[Result]:
         out = (Result * self.cfg.n_prn)()

@@ -13,6 +13,9 @@
  *              loops: [DLLBW DLLDamp DLLGain PLLBW PLLDamp PLLGain CorrelatorSpacing]; rec: 14 x n_periods x n,
  *              rows [P_i P_q E_i E_q L_i L_q PLLdiscri DLLdiscri remChip codeFreq carrierFreq remPhase
  *              sample_end numSample] (trackingCT.m:153-172)
+ *   [rec, I, Q] = gnssacq_mex('track', channels, cfg, loops, n_periods, spacing)   the same loop, and every period the
+ *              correlator bank at spacing (1 x n_taps, trackingCT_POS_updated_multicorrelator.m:41,207-260); I, Q:
+ *              n_taps x n_periods x n.  The bank only observes: rec is what the 5-argument form returns
  *              gnssacq_mex('close')                                         destroy the handles now
  *
  * `raw` is the block acquisition.m:29/34 reads, passed as int8 (or int16) WITHOUT conversion to
@@ -272,9 +275,11 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         gnssacq_track_record* rec;
         gnssacq_loop_params loops;
         mwSize dims[3];
-        double* out;
-        if (nrhs != 5 || !mxIsDouble(prhs[1]) || mxGetM(prhs[1]) != 7 || mxGetNumberOfElements(prhs[3]) != 7)
-            fail(GNSSACQ_ERR_INVALID_ARG, "track: (channels 7 x n, cfg, loops 1 x 7, n_periods)");
+        double *out, *bi = NULL, *bq = NULL;
+        int n_taps = 0;
+        if ((nrhs != 5 && nrhs != 6) || !mxIsDouble(prhs[1]) || mxGetM(prhs[1]) != 7 || mxGetNumberOfElements(prhs[3]) != 7 ||
+            (nrhs == 6 && !mxIsDouble(prhs[5])))
+            fail(GNSSACQ_ERR_INVALID_ARG, "track: (channels 7 x n, cfg, loops 1 x 7, n_periods[, spacing 1 x n_taps])");
         lp = mxGetPr(prhs[3]);
         n_ch = (int)mxGetN(prhs[1]);
         n_per = (int)mxGetScalar(prhs[4]);
@@ -284,7 +289,19 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         ch = (gnssacq_channel*)mxMalloc(sizeof(gnssacq_channel) * (size_t)(n_ch + 1));
         rec = (gnssacq_track_record*)mxMalloc(sizeof(gnssacq_track_record) * ((size_t)n_ch * (size_t)n_per + 1));
         channels_from(prhs[1], ch, n_ch, 0);
-        rc = gnssacq_track(g_handle[0], n_ch, ch, &loops, n_per, rec);
+        if (nrhs == 6) {                               /* I, Q: [channel][period][tap] = n_taps x n_periods x n */
+            n_taps = (int)mxGetNumberOfElements(prhs[5]);
+            dims[0] = (mwSize)n_taps; dims[1] = (mwSize)n_per; dims[2] = (mwSize)n_ch;
+            if (nlhs > 1) { plhs[1] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL); bi = mxGetPr(plhs[1]); }
+            else bi = (double*)mxMalloc(sizeof(double) * ((size_t)n_taps * n_per * n_ch + 1));
+            if (nlhs > 2) { plhs[2] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL); bq = mxGetPr(plhs[2]); }
+            else bq = (double*)mxMalloc(sizeof(double) * ((size_t)n_taps * n_per * n_ch + 1));
+            rc = gnssacq_track_bank(g_handle[0], n_ch, ch, &loops, n_per, n_taps, mxGetPr(prhs[5]), rec, bi, bq);
+            if (nlhs <= 1) mxFree(bi);
+            if (nlhs <= 2) mxFree(bq);
+        } else {
+            rc = gnssacq_track(g_handle[0], n_ch, ch, &loops, n_per, rec);
+        }
         if (rc != GNSSACQ_OK) { mxFree(ch); mxFree(rec); fail(rc, gnssacq_last_error(g_handle[0])); }
         dims[0] = 14; dims[1] = (mwSize)n_per; dims[2] = (mwSize)n_ch;
         plhs[0] = mxCreateNumericArray(3, dims, mxDOUBLE_CLASS, mxREAL);

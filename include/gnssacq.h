@@ -310,6 +310,20 @@ int gnssacq_loop_params_default(gnssacq_loop_params* p);
 int gnssacq_track(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start, const gnssacq_loop_params* loops,
                   int32_t n_periods, gnssacq_track_record* out);
 
+/* gnssacq_track, and every period also the correlator bank at spacing_chips[0..n_taps) (the 25-tap bank of
+ * trackingCT_POS_updated_multicorrelator.m:41,207-260, the 29-point grid of trackingVT_POS_updated.m:29).  The bank
+ * only observes: the loop is driven by E/P/L exactly as in gnssacq_track, and out[] is byte-identical to what
+ * gnssacq_track returns for the same arguments.  Tap t of period i of channel c is the gnssacq_correlate sum for that
+ * period's channel state and samples (same code-index rule, same int16 per-period DC removal):
+ *   bank_i[(c*n_periods + i)*n_taps + t], bank_q[...]
+ * Errors are those of gnssacq_track, plus GNSSACQ_ERR_INVALID_ARG for n_taps outside 1..32, a NULL spacing_chips,
+ * bank_i or bank_q, or a non-finite spacing.  The device keeps a 2 * n_channels * n_periods * n_taps double buffer
+ * (it grows; 64 channels x 100 000 periods x 32 taps = 3.3 GB): GNSSACQ_ERR_NOMEM when it cannot be allocated. */
+int gnssacq_track_bank(gnssacq_handle* h, int32_t n_channels, const gnssacq_channel* start,
+                       const gnssacq_loop_params* loops, int32_t n_periods,
+                       int32_t n_taps, const double* spacing_chips,
+                       gnssacq_track_record* out, double* bank_i, double* bank_q);
+
 /* Fine-frequency stage (replaces acquisition.m:89-121; SURVEY 8f-1).  `if_long` is the (L+1) ms block
  * acquisition.m:91/96 reads from the same file offset (host memory); for each of the n_sv acquired SVs
  * (prn[i], code_phase[i] = Acquired.codedelay) the code-stripped L ms are zero-padded to
