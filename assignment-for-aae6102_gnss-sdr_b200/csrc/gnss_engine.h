@@ -52,6 +52,7 @@ struct Geo {
     // column id (c', pos) -> b' (pos = 25*k1 + k2 holds b' = k1 + 5*k2)
     GNSS_HD static int bprime_of_pos(int pos) { return pos / 25 + 5 * (pos % 25); }
     GNSS_HD static int pos_of_bprime(int bp) { return 25 * (bp % 5) + bp / 5; }
+    GNSS_HD static bool valid(int col) { return col < ROW; }   // (columns >= ROW: a CTA's slice past the row's end)
     // output lag / frequency index of (a', column)
     GNSS_HD static int lag_of(int ap, int col) {
         const int cp = col / 125, pos = col - cp * 125;
@@ -116,6 +117,16 @@ struct Split {
     static constexpr int P3_TASKS = NR * 5;
     static constexpr int P4_TASKS = CH / 2;                // column PAIRS
 };
+
+// A search row's power accumulator as the row end reads it: [16 a'][CH] floats per CTA, CTA r holding columns
+// r*CH .. r*CH + CH-1 of geometry G, which says which columns hold a lag (valid) and maps lags to cells and back.
+template <class G_, int CH_>
+struct AccLayout {
+    using G = G_;
+    static constexpr int CH = CH_;
+};
+template <int Q, int R> using RowAcc = AccLayout<Geo<Q>, Split<Q, R>::CH>;       // search_kernel, search_kernel_l2x
+template <int Q, int R> using XchgAcc = AccLayout<GeoX<Q>, SplitX<Q, R>::CHX>;  // search_kernel_coop (XT layout)
 
 // ------------------------------------------------------------------ pass 1
 // compute half: load (functor) + DFT-Q over c, result left in registers
@@ -481,6 +492,19 @@ struct CodeLoader {
     }
 };
 
+// ---- IF sample idx of a block as (I, Q) (acquisition.m:27-32): int16 I/Q less the means, int8 I/Q, int8 real ----
+GNSS_HD cf if_sample(const void* raw, long long idx, int data_type, int precision, float mean_i, float mean_q) {
+    if (precision == 2) {
+        const int16_t* p = (const int16_t*)raw;
+        return mk((float)p[2 * idx] - mean_i, (float)p[2 * idx + 1] - mean_q);
+    }
+    if (data_type == 2) {
+        const int8_t* p = (const int8_t*)raw;
+        return mk((float)p[2 * idx], (float)p[2 * idx + 1]);
+    }
+    return mk((float)((const int8_t*)raw)[idx], 0.f);
+}
+
 // ---- wipe-off loader (K1): acquisition.m:43,56 with exact phase, plus the M-ms fold (A.8) ----
 GNSS_HD void carrier_sincos(double f_hz, double fs_hz, long long n1 /*1-based sample index*/,
                             float& co, float& si) {
@@ -496,6 +520,8 @@ GNSS_HD void carrier_sincos(double f_hz, double fs_hz, long long n1 /*1-based sa
 #endif
 }
 
+// Each ms holds n_ms = N - pad samples and is the start of an N-point transform: inputs n >= n_ms are zero padding
+// (none at a built N, pad = 0).  The carrier phase is that of sample j*n_ms + n + 1 of the coherent block.
 struct WipeoffLoader {
     static constexpr bool kStreams = false;
     const void* __restrict__ raw;   // start of this coherent block (sample 0 of the block)
@@ -504,32 +530,24 @@ struct WipeoffLoader {
     int coh_ms;                     // M
     double f_hz, fs_hz;             // IF + doppler of this base, Fs
     float mean_i, mean_q;           // int16 path only (acquisition.m:32)
+    int pad = 0;                    // zero inputs after each ms's samples
     template <int Q>
     GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
-        constexpr int N = Geo<Q>::N;
+        const int n_ms = Geo<Q>::N - pad;    // samples per ms: the fold's stride
         static_for<0, Q>([&](auto c_) {
             constexpr int C = decltype(c_)::value;
             const int n = Geo<Q>::good(a, b, C);
             float ax = 0.f, ay = 0.f;
-            for (int j = 0; j < coh_ms; ++j) {
-                const long long idx = (long long)j * N + n;
-                float xi, xq;
-                if (precision == 2) {
-                    const int16_t* p = (const int16_t*)raw;
-                    xi = (float)p[2 * idx] - mean_i;
-                    xq = (float)p[2 * idx + 1] - mean_q;
-                } else if (data_type == 2) {
-                    const int8_t* p = (const int8_t*)raw;
-                    xi = (float)p[2 * idx];
-                    xq = (float)p[2 * idx + 1];
-                } else {
-                    xi = (float)((const int8_t*)raw)[idx];
-                    xq = 0.f;
+            if (n < n_ms) {
+                for (int j = 0; j < coh_ms; ++j) {
+                    const long long idx = (long long)j * n_ms + n;
+                    const cf x = if_sample(raw, idx, data_type, precision, mean_i, mean_q);
+                    float co, si;
+                    carrier_sincos(f_hz, fs_hz, idx + 1, co, si);
+                    // explicit fmaf: which product is fused decides the rounding, so it must not be left to the compiler
+                    ax += fmaf(x.x, co, -(x.y * si));
+                    ay += fmaf(x.x, si, x.y * co);
                 }
-                float co, si;
-                carrier_sincos(f_hz, fs_hz, idx + 1, co, si);
-                ax += xi * co - xq * si;
-                ay += xi * si + xq * co;
             }
             z[C] = mk(ax, ay);
         });
@@ -553,23 +571,9 @@ struct FineLoader {
     // decimated sample n1 (of N), code-stripped and modulated for residue r
     GNSS_HD cf sample(int n1) const {
         const long long n = (long long)L * n1 + n2;
-        const long long idx = (long long)start + n;
-        float xi, xq;
-        if (precision == 2) {
-            const int16_t* p = (const int16_t*)raw;
-            xi = (float)p[2 * idx] - mean_i;
-            xq = (float)p[2 * idx + 1] - mean_q;
-        } else if (data_type == 2) {
-            const int8_t* p = (const int8_t*)raw;
-            xi = (float)p[2 * idx];
-            xq = (float)p[2 * idx + 1];
-        } else {
-            xi = (float)((const int8_t*)raw)[idx];
-            xq = 0.f;
-        }
+        const cf x = if_sample(raw, (long long)start + n, data_type, precision, mean_i, mean_q);
         const float cv = (float)ca[chip[n]];
-        xi *= cv;
-        xq *= cv;
+        const float xi = x.x * cv, xq = x.y * cv;
         const long long m = (n * (long long)r) % F;          // exact phase numerator
         const double fr = (double)m / (double)F;
         float co, si;
@@ -587,49 +591,6 @@ struct FineLoader {
         static_for<0, Q>([&](auto c_) {
             constexpr int C = decltype(c_)::value;
             z[C] = sample(Geo<Q>::good(a, b, C));
-        });
-    }
-};
-
-// ---- zero-padded shapes: each ms of n_ms < N samples is the start of an N-point transform ----
-// K1 (acquisition.m:43,56): WipeoffLoader with the fold's stride and the sample count per ms taken at run time;
-// inputs n >= n_ms are the zero padding.  The carrier phase is that of sample j*n_ms + n + 1 of the coherent block.
-struct PadWipeoffLoader {
-    static constexpr bool kStreams = false;
-    const void* __restrict__ raw;   // start of this coherent block
-    int data_type, precision, coh_ms;
-    int n_ms;                       // samples per ms
-    double f_hz, fs_hz;
-    float mean_i, mean_q;
-    template <int Q>
-    GNSS_HD void load(int a, int b, cf (&z)[Q]) const {
-        static_for<0, Q>([&](auto c_) {
-            constexpr int C = decltype(c_)::value;
-            const int n = Geo<Q>::good(a, b, C);
-            float ax = 0.f, ay = 0.f;
-            if (n < n_ms) {
-                for (int j = 0; j < coh_ms; ++j) {
-                    const long long idx = (long long)j * n_ms + n;
-                    float xi, xq;
-                    if (precision == 2) {
-                        const int16_t* p = (const int16_t*)raw;
-                        xi = (float)p[2 * idx] - mean_i;
-                        xq = (float)p[2 * idx + 1] - mean_q;
-                    } else if (data_type == 2) {
-                        const int8_t* p = (const int8_t*)raw;
-                        xi = (float)p[2 * idx];
-                        xq = (float)p[2 * idx + 1];
-                    } else {
-                        xi = (float)((const int8_t*)raw)[idx];
-                        xq = 0.f;
-                    }
-                    float co, si;
-                    carrier_sincos(f_hz, fs_hz, idx + 1, co, si);
-                    ax += xi * co - xq * si;
-                    ay += xi * si + xq * co;
-                }
-            }
-            z[C] = mk(ax, ay);
         });
     }
 };

@@ -49,7 +49,7 @@ struct WipeArgs {
     const void* raw;       // device IF block
     int data_type, precision, coh_ms, K;
     size_t block_bytes;    // bytes per coherent block
-    int n_ms;              // samples per ms (the fold's stride); < N: wipe_pad_kernel zero-pads each ms to the transform length
+    int n_ms;              // samples per ms (the fold's stride); < N: each ms is zero-padded to the transform length
     const double* base_freq_hz;   // [n_bases] IF + doppler of each base
     double fs_hz;
     const double* means;   // [2] int16 path (device), else nullptr
@@ -111,7 +111,7 @@ struct VariantOps {
     size_t smem_search, smem_transform;
     cudaError_t (*prepare)();
     cudaError_t (*launch_code)(const CodeArgs&, int units, cudaStream_t);
-    cudaError_t (*launch_wipe)(const WipeArgs&, int units, cudaStream_t);
+    cudaError_t (*launch_wipe)(const WipeArgs&, int units, cudaStream_t);     // K1 gathered from the IF block
     cudaError_t (*launch_wipe2)(const Wipe2Args&, int units, cudaStream_t);
     size_t (*smem_wipe2)(int pitch, int coh_ms);
     cudaError_t (*launch_natural)(const NaturalArgs&, int units, cudaStream_t);
@@ -125,8 +125,7 @@ struct VariantOps {
     cudaError_t (*launch_search_coop)(const SearchArgs&, int groups, cudaStream_t);
     int (*max_groups_coop)();              // co-resident CTA groups on the current device
     size_t partial_bytes_per_group;        // coop variant: one power plane (all R slices) of the tail hand-over
-    // zero-padded shapes (samples per ms < N): K1 gather kernel, and the three stages of a Bluestein DFT
-    cudaError_t (*launch_wipe_pad)(const WipeArgs&, int units, cudaStream_t);
+    // zero-padded shapes (samples per ms < N): the three stages of a Bluestein DFT
     cudaError_t (*launch_chirp_in)(const ChirpArgs&, int units, cudaStream_t);       // ChirpArgs.in -> v
     cudaError_t (*launch_fine_chirp)(const FineArgs&, const ChirpArgs&, int units, cudaStream_t);   // fine samples -> v
     cudaError_t (*launch_chirp_out)(const ChirpArgs&, int units, cudaStream_t);      // v -> out

@@ -1,12 +1,16 @@
 // gnss_kernels.cuh -- sm_100a kernels around the engine passes (gnss_engine.h).
 //
-//   code_kernel    K0  fft(code replica) -> conj(.)/N, G layout          (acquisition.m:58, once per handle)
-//   wipe_kernel    K1  wipe-off (+ M-ms fold) + forward FFT per (base, block)   (acquisition.m:56-57)
-//   search_kernel  K2  per (PRN, bin) row: for each of the K blocks multiply the two spectra in the
-//                      load stage, transform, |.|^2, accumulate on chip; then K3 = row peak, first-index
-//                      argmax, sum of squares and windowed sum of squares   (acquisition.m:59,62-63,67)
-//   natural_kernel     plain forward DFT (test hook)
-//   wipe_pad_kernel, chirp_*_kernel   K1 and the Bluestein N-point DFTs of a shape zero-padded into the transform
+//   code_kernel      K0  fft(code replica) -> conj(.)/N, G layout          (acquisition.m:58, once per handle)
+//   wipe_pad_kernel  K1  wipe-off (+ M-ms fold, + zero padding of each ms) + forward FFT per (base, block),
+//                        gathered from the IF block   (acquisition.m:56-57); wipe2_kernel: the same from comb rows
+//   search_kernel    K2  per (PRN, bin) row: for each of the K blocks multiply the two spectra in the
+//                        load stage, transform, |.|^2, accumulate on chip; then K3 = row peak, first-index
+//                        argmax, sum of squares and windowed sum of squares   (acquisition.m:59,62-63,67)
+//                        (search_kernel_l2x, search_kernel_coop: the same with other exchanges; all three
+//                        share row_coords, row_loader, row_scan and window_sum, the two cluster kernels
+//                        cluster_row_end)
+//   natural_kernel       plain forward DFT (test hook)
+//   chirp_*_kernel       the Bluestein N-point DFTs of a shape zero-padded into the transform
 //
 // One transform = one thread-block cluster of R CTAs; each CTA keeps 16/R rows of the
 // [16][Q][125] prime-factor array in shared memory, pass 4 pulls the other CTAs' rows through
@@ -29,18 +33,6 @@ struct NaturalLoader {
         static_for<0, Q>([&](auto c_) {
             constexpr int C = decltype(c_)::value;
             z[C] = in[Geo<Q>::good(a, b, C)];
-        });
-    }
-};
-struct NaturalStorer {
-    cf* __restrict__ out;
-    template <int Q, int R>
-    __device__ __forceinline__ void store2(int col, int, const cf (&w0)[16], const cf (&w1)[16]) {
-        static_for<0, 16>([&](auto i_) {
-            constexpr int I = decltype(i_)::value;
-            constexpr int AP = (I / 4) + 4 * (I % 4);
-            out[Geo<Q>::lag_of(AP, col)] = w0[I];
-            if (col + 1 < Geo<Q>::ROW) out[Geo<Q>::lag_of(AP, col + 1)] = w1[I];
         });
     }
 };
@@ -181,6 +173,109 @@ __device__ __forceinline__ void unit_device_pipelined(const Loader& ld, Storer& 
     cl_arrive<R>();
 }
 
+// ---- the search row: its PRN index, bin and block-0 loader; the row end (K3) over an accumulator layout ----
+// Launch row lrow -> PRN index p, bin b: row = bin * P + prn_index (PRN fastest: rows in flight share the same
+// forward spectra in L2)
+__device__ __forceinline__ void row_coords(const SearchArgs& a, int lrow, int& p, int& b) {
+    const int row = a.rows ? a.rows[lrow] : a.row_first + lrow;
+    p = row % a.P;
+    b = row / a.P;
+}
+// loader of block 0 of row (p, b)
+template <int Q>
+__device__ __forceinline__ SearchLoader row_loader(const SearchArgs& a, int p, int b) {
+    using G = Geo<Q>;
+    int sa, sb, sc;
+    G::shift_coords(a.bin_shift[b], sa, sb, sc);
+    return SearchLoader{a.cc + (size_t)p * G::N, a.x + (size_t)a.bin_base[b] * a.K * G::NX, sa, sb, sc};
+}
+
+// Cell by cell over this CTA's slice: peak (first lag on ties), sum of squares, optional surface store of row (p, b).
+// Only lags below n_lags count (m >= n_lags: zero padding of a padded shape).
+template <class L, int T>
+__device__ __forceinline__ void row_scan(const SearchArgs& a, int p, int b, const float* acc, int rank, int tid,
+                                         float& bv, int& bm, double& ss) {
+    for (int e = tid; e < 16 * L::CH; e += T) {
+        const int ap = e / L::CH, t = e - ap * L::CH;
+        const int col = rank * L::CH + t;
+        if (L::G::valid(col)) {
+            const int m = L::G::lag_of(ap, col);
+            if (m < a.n_lags) {
+                const float v = acc[e];
+                if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
+                ss += (double)v * (double)v;
+                if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
+            }
+        }
+    }
+}
+
+// Sum of squares over lags gm-(w-1) .. gm+(w-1), clipped to [0, n_lags), of the cells in this CTA's slice
+template <class L, int T>
+__device__ __forceinline__ double window_sum(const SearchArgs& a, int gm, const float* acc, int rank, int tid) {
+    double wsum = 0.0;
+    for (int i = tid; i < 2 * a.w - 1; i += T) {
+        const int m = gm - (a.w - 1) + i;
+        if (m >= 0 && m < a.n_lags) {
+            int ap, col;
+            L::G::cell_of_lag(m, ap, col);
+            if (col / L::CH == rank) {
+                const float v = acc[ap * L::CH + (col - rank * L::CH)];
+                wsum += (double)v * (double)v;
+            }
+        }
+    }
+    return wsum;
+}
+
+// K3 of the two cluster kernels: scan, cluster-wide winner and sums through DSMEM, rank 0 stores the Candidate.
+// Ends with rank 0 reading the other CTAs' RedScratch: the caller's barrier must keep them alive until then.
+template <int Q, int R, int T>
+__device__ __forceinline__ void cluster_row_end(const SearchArgs& a, int p, int b, const float* acc, RedScratch* rs,
+                                                cg::cluster_group& cluster, int rank, int tid) {
+    using L = RowAcc<Q, R>;
+    float bv = -1.f;
+    int bm = INT_MAX;
+    double ss = 0.0;
+    row_scan<L, T>(a, p, b, acc, rank, tid, bv, bm, ss);
+    block_reduce<T>(bv, bm, ss, rs);
+    if (tid == 0) { rs->peak = bv; rs->lag = bm; rs->sum_all = ss; }
+    if constexpr (R > 1) cluster.sync(); else __syncthreads();
+    if (tid == 0) {
+        float gv = -1.f;
+        int gm = INT_MAX;
+        for (int r = 0; r < R; ++r) {
+            const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
+            const float ov = o->peak;
+            const int om = o->lag;
+            if (peak_better(ov, om, gv, gm)) { gv = ov; gm = om; }
+        }
+        rs->g_peak = gv;
+        rs->g_lag = gm;
+    }
+    __syncthreads();
+    double wsum = window_sum<L, T>(a, rs->g_lag, acc, rank, tid);
+    float dv = -1.f;
+    int dm = INT_MAX;
+    block_reduce<T>(dv, dm, wsum, rs);
+    if (tid == 0) rs->sum_win = wsum;
+    if constexpr (R > 1) cluster.sync(); else __syncthreads();
+    if (rank == 0 && tid == 0) {
+        double s_all = 0.0, s_win = 0.0;
+        for (int r = 0; r < R; ++r) {
+            const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
+            s_all += o->sum_all;
+            s_win += o->sum_win;
+        }
+        Candidate c;
+        c.peak = rs->g_peak;
+        c.lag = rs->g_lag;
+        c.sum_all = s_all;
+        c.sum_win = s_win;
+        a.cand[(size_t)p * a.cand_stride + b] = c;
+    }
+}
+
 #define GNSS_KERNEL_PROLOGUE                                                     \
     using S = Split<Q, R>;                                                       \
     using G = Geo<Q>;                                                            \
@@ -206,8 +301,10 @@ __global__ void __launch_bounds__(T, MINB) code_kernel(CodeArgs a) {
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
 
+// K1 gathered from the IF block (acquisition.m:43,56-57): every shape that has no comb rows, each ms of n_ms
+// samples zero-padded to the transform length (no padding at a built N: n_ms = N)
 template <int Q, int R, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) wipe_kernel(WipeArgs a) {
+__global__ void __launch_bounds__(T, MINB) wipe_pad_kernel(WipeArgs a) {
     GNSS_KERNEL_PROLOGUE
     Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
     fill_tw125(tw, tid, T);
@@ -222,6 +319,7 @@ __global__ void __launch_bounds__(T, MINB) wipe_kernel(WipeArgs a) {
     ld.fs_hz = a.fs_hz;
     ld.mean_i = a.means ? (float)a.means[0] : 0.f;
     ld.mean_q = a.means ? (float)a.means[1] : 0.f;
+    ld.pad = G::N - a.n_ms;
     SpectrumStorer st{a.x + (size_t)unit * G::NX, 1.0f, 0, 1};
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
@@ -334,17 +432,12 @@ __global__ void __launch_bounds__(T, MINB) natural_kernel(NaturalArgs a) {
     fill_tw125(tw, tid, T);
     __syncthreads();
     NaturalLoader ld{a.in + (size_t)unit * G::N};
-    NaturalStorer st{a.out + (size_t)unit * G::N};
+    NaturalStorerHD st{a.out + (size_t)unit * G::N};
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
 
-// fine-frequency transforms: unit = ((sv * K) + r) * L + n2
-template <int Q, int R, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) fine_kernel(FineArgs a) {
-    GNSS_KERNEL_PROLOGUE
-    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
-    fill_tw125(tw, tid, T);
-    __syncthreads();
+// the samples of fine-frequency transform unit = ((sv * K) + r) * L + n2
+__device__ __forceinline__ FineLoader fine_loader(const FineArgs& a, int unit) {
     const int n2 = unit % a.L, r = (unit / a.L) % a.K, sv = unit / (a.L * a.K);
     FineLoader ld;
     ld.raw = a.raw;
@@ -359,33 +452,21 @@ __global__ void __launch_bounds__(T, MINB) fine_kernel(FineArgs a) {
     ld.n2 = n2;
     ld.r = r;
     ld.F = a.F;
+    return ld;
+}
+
+template <int Q, int R, int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) fine_kernel(FineArgs a) {
+    GNSS_KERNEL_PROLOGUE
+    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
+    fill_tw125(tw, tid, T);
+    __syncthreads();
+    const FineLoader ld = fine_loader(a, unit);
     NaturalStorerHD st{a.u + (size_t)unit * G::N};
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
 
 // ---- zero-padded shapes (samples per ms < N) ----
-// K1 for a padded shape: wipe_kernel with the fold stride and the zero padding of PadWipeoffLoader
-template <int Q, int R, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) wipe_pad_kernel(WipeArgs a) {
-    GNSS_KERNEL_PROLOGUE
-    Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
-    fill_tw125(tw, tid, T);
-    __syncthreads();
-    const int base = unit / a.K, k = unit - base * a.K;
-    PadWipeoffLoader ld;
-    ld.raw = (const unsigned char*)a.raw + (size_t)k * a.block_bytes;
-    ld.data_type = a.data_type;
-    ld.precision = a.precision;
-    ld.coh_ms = a.coh_ms;
-    ld.n_ms = a.n_ms;
-    ld.f_hz = a.base_freq_hz[base];
-    ld.fs_hz = a.fs_hz;
-    ld.mean_i = a.means ? (float)a.means[0] : 0.f;
-    ld.mean_q = a.means ? (float)a.means[1] : 0.f;
-    SpectrumStorer st{a.x + (size_t)unit * G::NX, 1.0f, 0, 1};
-    unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
-}
-
 // Bluestein stage 1 of gnssacq_fft_forward: v[unit] = FFT_N(conj(ch) * in[unit], zero-padded)
 template <int Q, int R, int T, int MINB>
 __global__ void __launch_bounds__(T, MINB) chirp_in_kernel(ChirpArgs c) {
@@ -405,21 +486,7 @@ __global__ void __launch_bounds__(T, MINB) fine_chirp_kernel(FineArgs a, ChirpAr
     Tw4* tw = reinterpret_cast<Tw4*>(D + S::D_ELEMS);
     fill_tw125(tw, tid, T);
     __syncthreads();
-    const int n2 = unit % a.L, r = (unit / a.L) % a.K, sv = unit / (a.L * a.K);
-    FineLoader f;
-    f.raw = a.raw;
-    f.chip = a.chip;
-    f.ca = a.ca + (size_t)sv * 1023;
-    f.data_type = a.data_type;
-    f.precision = a.precision;
-    f.mean_i = a.means ? (float)a.means[0] : 0.f;
-    f.mean_q = a.means ? (float)a.means[1] : 0.f;
-    f.start = a.start[sv];
-    f.L = a.L;
-    f.n2 = n2;
-    f.r = r;
-    f.F = a.F;
-    ChirpLoader<FineLoader> ld{f, c.chirp, c.n};
+    ChirpLoader<FineLoader> ld{fine_loader(a, unit), c.chirp, c.n};
     NaturalStorerHD st{c.v + (size_t)unit * G::N};
     unit_device<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
 }
@@ -442,88 +509,24 @@ __global__ void __launch_bounds__(T, MINB) search_kernel(SearchArgs a) {
     float* acc = reinterpret_cast<float*>(D + S::D_ELEMS);
     Tw4* tw = reinterpret_cast<Tw4*>(acc + Smem<Q, R>::acc_floats);
     RedScratch* rs = reinterpret_cast<RedScratch*>(tw + 100);
-    const int row = a.rows ? a.rows[unit] : a.row_first + unit;   // row = bin * P + prn_index (PRN fastest: rows in
-    const int p = row % a.P, b = row / a.P;     // flight share the same forward spectra in L2)
+    int p, b;
+    row_coords(a, unit, p, b);
 
     fill_tw125(tw, tid, T);
     for (int e = tid; e < S::ACC_ELEMS; e += T) acc[e] = 0.f;
     __syncthreads();
 
-    int sa, sb, sc;
-    G::shift_coords(a.bin_shift[b], sa, sb, sc);
-    const cf* ccp = a.cc + (size_t)p * G::N;
-    const cf* xb = a.x + (size_t)a.bin_base[b] * a.K * G::NX;
+    const SearchLoader ld0 = row_loader<Q>(a, p, b);
     PowerAccumStorer st{acc};
     cl_arrive<R>();
     for (int k = 0; k < a.K; ++k) {
-        SearchLoader ld{ccp, xb + (size_t)k * G::NX, sa, sb, sc};
+        SearchLoader ld = ld0;
+        ld.x += (size_t)k * G::NX;
         unit_device_pipelined<Q, R, T>(ld, st, D, Dall, tw, rank, tid);
     }
     cl_wait<R>();
 
-    // ---- K3: row peak (first index on ties), sum of squares, windowed sum of squares ----
-    float bv = -1.f;
-    int bm = INT_MAX;
-    double ss = 0.0;
-    for (int e = tid; e < S::ACC_ELEMS; e += T) {
-        const int ap = e / S::CH, t = e - ap * S::CH;
-        const int col = rank * S::CH + t;
-        const int m = G::lag_of(ap, col);
-        if (col < S::ROW && m < a.n_lags) {         // (m >= n_lags: zero padding of a padded shape)
-            const float v = acc[e];
-            if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
-            ss += (double)v * (double)v;
-            if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
-        }
-    }
-    block_reduce<T>(bv, bm, ss, rs);
-    if (tid == 0) { rs->peak = bv; rs->lag = bm; rs->sum_all = ss; }
-    if constexpr (R > 1) cluster.sync(); else __syncthreads();
-    if (tid == 0) {
-        float gv = -1.f;
-        int gm = INT_MAX;
-        for (int r = 0; r < R; ++r) {
-            const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
-            const float ov = o->peak;
-            const int om = o->lag;
-            if (peak_better(ov, om, gv, gm)) { gv = ov; gm = om; }
-        }
-        rs->g_peak = gv;
-        rs->g_lag = gm;
-    }
-    __syncthreads();
-    const int gm = rs->g_lag;
-    double wsum = 0.0;
-    for (int i = tid; i < 2 * a.w - 1; i += T) {
-        const int m = gm - (a.w - 1) + i;
-        if (m >= 0 && m < a.n_lags) {
-            int ap, col;
-            G::cell_of_lag(m, ap, col);
-            if (col / S::CH == rank) {
-                const float v = acc[ap * S::CH + (col - rank * S::CH)];
-                wsum += (double)v * (double)v;
-            }
-        }
-    }
-    float dv = -1.f;
-    int dm = INT_MAX;
-    block_reduce<T>(dv, dm, wsum, rs);
-    if (tid == 0) rs->sum_win = wsum;
-    if constexpr (R > 1) cluster.sync(); else __syncthreads();
-    if (rank == 0 && tid == 0) {
-        double s_all = 0.0, s_win = 0.0;
-        for (int r = 0; r < R; ++r) {
-            const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
-            s_all += o->sum_all;
-            s_win += o->sum_win;
-        }
-        Candidate c;
-        c.peak = rs->g_peak;
-        c.lag = rs->g_lag;
-        c.sum_all = s_all;
-        c.sum_win = s_win;
-        a.cand[(size_t)p * a.cand_stride + b] = c;
-    }
+    cluster_row_end<Q, R, T>(a, p, b, acc, rs, cluster, rank, tid);
     if constexpr (R > 1) cluster.sync();   // keep every CTA's shared memory alive until rank 0 has read it
 }
 
@@ -546,17 +549,11 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
     PowerAccumStorer st{acc};
 
     for (int lrow = slot; lrow < a.n_rows; lrow += ncl) {
-        const int row = a.rows ? a.rows[lrow] : a.row_first + lrow;
-        const int p = row % a.P, b = row / a.P;
+        int p, b;
+        row_coords(a, lrow, p, b);
+        const SearchLoader ld0 = row_loader<Q>(a, p, b);
         for (int e = tid; e < S::ACC_ELEMS; e += T) acc[e] = 0.f;
-        int sa, sb, sc;
-        G::shift_coords(a.bin_shift[b], sa, sb, sc);
-        const cf* ccp = a.cc + (size_t)p * G::N;
-        const cf* xb = a.x + (size_t)a.bin_base[b] * a.K * G::NX;
-        {
-            SearchLoader ld{ccp, xb, sa, sb, sc};
-            for (int t = tid; t < S::P1_TASKS; t += T) pass1_task<Q, R>(t, rank, ld, D);
-        }
+        for (int t = tid; t < S::P1_TASKS; t += T) pass1_task<Q, R>(t, rank, ld0, D);
         __syncthreads();
         pass2_all<Q, R, T>(D, tw, tid);
         __syncthreads();
@@ -574,7 +571,8 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
                 for (int i = tid; i < S::D_ELEMS / 2; i += T) dst[i] = src[i];
             }
             if (more) {
-                SearchLoader ld{ccp, xb + (size_t)(k + 1) * G::NX, sa, sb, sc};
+                SearchLoader ld = ld0;
+                ld.x += (size_t)(k + 1) * G::NX;
                 cf z[Q];
                 const bool has = tid < S::P1_TASKS;
                 if (has) pass1_compute<Q, R>(tid, rank, ld, z);
@@ -596,69 +594,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_l2x(SearchArgs a) {
         }
         __syncthreads();
 
-        // ---- K3 (identical to search_kernel) ----
-        float bv = -1.f;
-        int bm = INT_MAX;
-        double ss = 0.0;
-        for (int e = tid; e < S::ACC_ELEMS; e += T) {
-            const int ap = e / S::CH, t = e - ap * S::CH;
-            const int col = rank * S::CH + t;
-            const int m = G::lag_of(ap, col);
-            if (col < S::ROW && m < a.n_lags) {         // (m >= n_lags: zero padding of a padded shape)
-                const float v = acc[e];
-                if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
-                ss += (double)v * (double)v;
-                if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
-            }
-        }
-        block_reduce<T>(bv, bm, ss, rs);
-        if (tid == 0) { rs->peak = bv; rs->lag = bm; rs->sum_all = ss; }
-        if constexpr (R > 1) cluster.sync(); else __syncthreads();
-        if (tid == 0) {
-            float gv = -1.f;
-            int gm = INT_MAX;
-            for (int r = 0; r < R; ++r) {
-                const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
-                const float ov = o->peak;
-                const int om = o->lag;
-                if (peak_better(ov, om, gv, gm)) { gv = ov; gm = om; }
-            }
-            rs->g_peak = gv;
-            rs->g_lag = gm;
-        }
-        __syncthreads();
-        const int gm = rs->g_lag;
-        double wsum = 0.0;
-        for (int i = tid; i < 2 * a.w - 1; i += T) {
-            const int m = gm - (a.w - 1) + i;
-            if (m >= 0 && m < a.n_lags) {
-                int ap, col;
-                G::cell_of_lag(m, ap, col);
-                if (col / S::CH == rank) {
-                    const float v = acc[ap * S::CH + (col - rank * S::CH)];
-                    wsum += (double)v * (double)v;
-                }
-            }
-        }
-        float dv = -1.f;
-        int dm = INT_MAX;
-        block_reduce<T>(dv, dm, wsum, rs);
-        if (tid == 0) rs->sum_win = wsum;
-        if constexpr (R > 1) cluster.sync(); else __syncthreads();
-        if (rank == 0 && tid == 0) {
-            double s_all = 0.0, s_win = 0.0;
-            for (int r = 0; r < R; ++r) {
-                const RedScratch* o = (R > 1) ? cluster.map_shared_rank(rs, r) : rs;
-                s_all += o->sum_all;
-                s_win += o->sum_win;
-            }
-            Candidate c;
-            c.peak = rs->g_peak;
-            c.lag = rs->g_lag;
-            c.sum_all = s_all;
-            c.sum_win = s_win;
-            a.cand[(size_t)p * a.cand_stride + b] = c;
-        }
+        cluster_row_end<Q, R, T>(a, p, b, acc, rs, cluster, rank, tid);
         if constexpr (R > 1) cluster.sync(); else __syncthreads();   // slots are rewritten by the next row
     }
 }
@@ -799,11 +735,9 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
     };
     const int n_rows = a.n_rows;              // the launch's rows: a.rows[0 .. n_rows), or [row_first, row_first + n_rows)
     auto loader_of = [&](int lrow) {          // loader of block 0 of a row (two or three dependent table reads: once per row)
-        const int row = a.rows ? a.rows[lrow] : a.row_first + lrow;
-        const int p = row % a.P, b = row / a.P;
-        int sa, sb, sc;
-        G::shift_coords(a.bin_shift[b], sa, sb, sc);
-        return SearchLoader{a.cc + (size_t)p * G::N, a.x + (size_t)a.bin_base[b] * a.K * G::NX, sa, sb, sc};
+        int p, b;
+        row_coords(a, lrow, p, b);
+        return row_loader<Q>(a, p, b);
     };
     // Schedule.  floor(n_rows / ngroups) full rounds of whole rows, strided (row = round*ngroups + group: at
     // any time the groups work on neighbouring rows, i.e. on the same forward spectra -- contiguous row ranges
@@ -958,24 +892,13 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
                                       a.K - cp.ke, tid);
                 __syncthreads();
             }
-            const int grow = a.rows ? a.rows[row] : a.row_first + row, p = grow % a.P, b = grow / a.P;
+            int p, b;
+            row_coords(a, row, p, b);
             float bv = -1.f;
             int bm = INT_MAX;
             double ss = 0.0;
             if (a.surface || a.n_lags < G::N) {   // debug path and padded shapes: every cell's lag is needed
-                for (int e = tid; e < SX::ACC_ELEMS; e += T) {
-                    const int ap = e / SX::CHX, t = e - ap * SX::CHX;
-                    const int ex = rank * SX::CHX + t;
-                    if (GX::valid(ex)) {
-                        const int m = GX::lag_of(ap, ex);
-                        if (m < a.n_lags) {        // (m >= n_lags: zero padding of a padded shape)
-                            const float v = acc[e];
-                            if (peak_better(v, m, bv, bm)) { bv = v; bm = m; }
-                            ss += (double)v * (double)v;
-                            if (a.surface) a.surface[((size_t)p * a.B + b) * a.n_lags + m] = v;
-                        }
-                    }
-                }
+                row_scan<XchgAcc<Q, R>, T>(a, p, b, acc, rank, tid, bv, bm, ss);
             } else {
                 // The lag of a cell costs ~40 integer instructions (two divisions, a CRT): only compute it
                 // for cells that can still win.  The padding columns hold exact zeros (their inputs are never
@@ -1019,19 +942,7 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
                 rs->g_lag = gm;
             }
             __syncthreads();
-            const int gm = rs->g_lag;
-            double wsum = 0.0;
-            for (int i = tid; i < 2 * a.w - 1; i += T) {
-                const int m = gm - (a.w - 1) + i;
-                if (m >= 0 && m < a.n_lags) {
-                    int ap, ex;
-                    GX::cell_of_lag(m, ap, ex);
-                    if (ex / SX::CHX == rank) {
-                        const float v = acc[ap * SX::CHX + (ex - rank * SX::CHX)];
-                        wsum += (double)v * (double)v;
-                    }
-                }
-            }
+            double wsum = window_sum<XchgAcc<Q, R>, T>(a, rs->g_lag, acc, rank, tid);
             float dv = -1.f;
             int dm = INT_MAX;
             block_reduce<T>(dv, dm, wsum, rs);
@@ -1075,22 +986,27 @@ __global__ void __launch_bounds__(T, MINB) search_kernel_coop(SearchArgs a) {
 }
 
 // ------------------------------------------------------------------ launch glue
-template <class K, class A>
-static cudaError_t launch_clustered(K kern, const A& args, int units, int R, int T, size_t smem, cudaStream_t s) {
-    cudaLaunchConfig_t cfg = {};
+// `units` clusters of R CTAs of T threads; cfg points at attr
+static void cluster_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute& attr, int units, int R, int T, size_t smem,
+                           cudaStream_t s) {
+    cfg = {};
     cfg.gridDim = dim3((unsigned)(units * R), 1, 1);
     cfg.blockDim = dim3((unsigned)T, 1, 1);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)R;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = (unsigned)R;
+    attr.val.clusterDim.y = 1;
+    attr.val.clusterDim.z = 1;
+    cfg.attrs = &attr;
     cfg.numAttrs = 1;
-    A copy = args;
-    return cudaLaunchKernelEx(&cfg, kern, copy);
+}
+template <class K, class... A>
+static cudaError_t launch_clustered(K kern, int units, int R, int T, size_t smem, cudaStream_t s, const A&... args) {
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute attr;
+    cluster_config(cfg, attr, units, R, T, smem, s);
+    return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 
 template <int Q, int R, int T, int MINB>
@@ -1101,35 +1017,28 @@ struct Variant {
     static constexpr int TT = R > 8 ? 256 : T;
     static constexpr int MT = R > 8 ? 2 : MINB;
     static cudaError_t prepare() {
-        cudaError_t e;
-        e = cudaFuncSetAttribute(code_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wipe_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wipe2_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(natural_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(fine_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wipe_pad_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(chirp_in_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(fine_chirp_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(chirp_out_kernel<Q, RT, TT, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, RT>::transform);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(search_kernel_coop<Q, R, T, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, R>::search);
-        if (e != cudaSuccess) return e;
-
-        e = cudaFuncSetAttribute(search_kernel_l2x<Q, R, T, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, R>::search);
-        if (e != cudaSuccess) return e;
-        return cudaFuncSetAttribute(search_kernel<Q, R, T, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Smem<Q, R>::search);
+        const struct { const void* kernel; size_t smem; } k[] = {
+            {(const void*)code_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)wipe2_kernel<Q, RT, TT, MT>, (size_t)227 * 1024},
+            {(const void*)natural_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)fine_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)wipe_pad_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)chirp_in_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)fine_chirp_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)chirp_out_kernel<Q, RT, TT, MT>, Smem<Q, RT>::transform},
+            {(const void*)search_kernel_coop<Q, R, T, MINB>, Smem<Q, R>::search},
+            {(const void*)search_kernel_l2x<Q, R, T, MINB>, Smem<Q, R>::search},
+            {(const void*)search_kernel<Q, R, T, MINB>, Smem<Q, R>::search},
+        };
+        for (const auto& f : k) {
+            const cudaError_t e = cudaFuncSetAttribute(f.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f.smem);
+            if (e != cudaSuccess) return e;
+        }
+        return cudaSuccess;
     }
     static cudaError_t launch_search_l2x(const SearchArgs& a, int clusters, cudaStream_t s) {
         if (R > 8) return cudaErrorInvalidConfiguration;
-        return launch_clustered(search_kernel_l2x<Q, R, T, MINB>, a, clusters, R, T, Smem<Q, R>::search, s);
+        return launch_clustered(search_kernel_l2x<Q, R, T, MINB>, clusters, R, T, Smem<Q, R>::search, s, a);
     }
     static cudaError_t launch_search_coop(const SearchArgs& a, int groups, cudaStream_t s) {
         SearchArgs copy = a;
@@ -1145,68 +1054,43 @@ struct Variant {
         return per_sm * sms / R;
     }
     static int max_clusters_l2x() {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(R * 1024), 1, 1);
-        cfg.blockDim = dim3((unsigned)T, 1, 1);
-        cfg.dynamicSmemBytes = Smem<Q, R>::search;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)R;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
+        cudaLaunchConfig_t cfg;
+        cudaLaunchAttribute attr;
+        cluster_config(cfg, attr, 1024, R, T, Smem<Q, R>::search, 0);
         int n = 0;
         if (cudaOccupancyMaxActiveClusters(&n, search_kernel_l2x<Q, R, T, MINB>, &cfg) != cudaSuccess) { cudaGetLastError(); return 0; }
         return n;
     }
     static cudaError_t launch_code(const CodeArgs& a, int units, cudaStream_t s) {
-        return launch_clustered(code_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(code_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, a);
     }
     static cudaError_t launch_wipe(const WipeArgs& a, int units, cudaStream_t s) {
-        return launch_clustered(wipe_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(wipe_pad_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, a);
     }
     static size_t smem_wipe2(int pitch, int coh_ms) {
         return Smem<Q, RT>::transform + (size_t)(coh_ms > 1 ? 2 : 1) * Split<Q, RT>::A * (size_t)pitch;
     }
     static cudaError_t launch_wipe2(const Wipe2Args& a, int units, cudaStream_t s) {
-        return launch_clustered(wipe2_kernel<Q, RT, TT, MT>, a, units, RT, TT, smem_wipe2(a.pitch, a.coh_ms), s);
+        return launch_clustered(wipe2_kernel<Q, RT, TT, MT>, units, RT, TT, smem_wipe2(a.pitch, a.coh_ms), s, a);
     }
     static cudaError_t launch_natural(const NaturalArgs& a, int units, cudaStream_t s) {
-        return launch_clustered(natural_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(natural_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, a);
     }
     static cudaError_t launch_fine(const FineArgs& a, int units, cudaStream_t s) {
-        return launch_clustered(fine_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
-    }
-    static cudaError_t launch_wipe_pad(const WipeArgs& a, int units, cudaStream_t s) {
-        return launch_clustered(wipe_pad_kernel<Q, RT, TT, MT>, a, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(fine_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, a);
     }
     static cudaError_t launch_chirp_in(const ChirpArgs& c, int units, cudaStream_t s) {
-        return launch_clustered(chirp_in_kernel<Q, RT, TT, MT>, c, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(chirp_in_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, c);
     }
     static cudaError_t launch_fine_chirp(const FineArgs& a, const ChirpArgs& c, int units, cudaStream_t s) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)(units * RT), 1, 1);
-        cfg.blockDim = dim3((unsigned)TT, 1, 1);
-        cfg.dynamicSmemBytes = Smem<Q, RT>::transform;
-        cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)RT;
-        attr[0].val.clusterDim.y = 1;
-        attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        FineArgs fa = a;
-        ChirpArgs ca = c;
-        return cudaLaunchKernelEx(&cfg, fine_chirp_kernel<Q, RT, TT, MT>, fa, ca);
+        return launch_clustered(fine_chirp_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, a, c);
     }
     static cudaError_t launch_chirp_out(const ChirpArgs& c, int units, cudaStream_t s) {
-        return launch_clustered(chirp_out_kernel<Q, RT, TT, MT>, c, units, RT, TT, Smem<Q, RT>::transform, s);
+        return launch_clustered(chirp_out_kernel<Q, RT, TT, MT>, units, RT, TT, Smem<Q, RT>::transform, s, c);
     }
     static cudaError_t launch_search(const SearchArgs& a, int rows, cudaStream_t s) {
         if (R > 8) return cudaErrorInvalidConfiguration;       // DSMEM variant needs a portable cluster
-        return launch_clustered(search_kernel<Q, R, T, MINB>, a, rows, R, T, Smem<Q, R>::search, s);
+        return launch_clustered(search_kernel<Q, R, T, MINB>, rows, R, T, Smem<Q, R>::search, s, a);
     }
     static constexpr VariantOps ops() {
         return VariantOps{Q, R, T, Smem<Q, R>::search, Smem<Q, RT>::transform,
@@ -1215,7 +1099,7 @@ struct Variant {
                           (size_t)2 * 16 * (Split<Q, R>::RS > GeoX<Q>::RSX ? Split<Q, R>::RS : GeoX<Q>::RSX) * sizeof(cf),
                           &launch_search_coop, &max_groups_coop,
                           (size_t)R * SplitX<Q, R>::ACC_ELEMS * sizeof(float),
-                          &launch_wipe_pad, &launch_chirp_in, &launch_fine_chirp, &launch_chirp_out};
+                          &launch_chirp_in, &launch_fine_chirp, &launch_chirp_out};
     }
 };
 

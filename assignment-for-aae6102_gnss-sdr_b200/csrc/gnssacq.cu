@@ -487,22 +487,25 @@ int stage_and_upload(gnssacq_handle* h, void* d_dst, const void* host_src, cudaS
     return GNSSACQ_OK;
 }
 
+// int16 per-component means of n_pairs samples into h->d_means, summed over the `scan` (I, Q) pairs at `src`
+// (two launches)
+static int launch_means(gnssacq_handle* h, const void* src, long long scan, long long n_pairs, cudaStream_t s) {
+    CU(cudaMemsetAsync(h->d_sums.get(), 0, 2 * sizeof(long long), s));
+    sum_int16_kernel<<<296, 256, 0, s>>>((const int16_t*)src, scan, h->d_sums.get());
+    means_kernel<<<1, 1, 0, s>>>(h->d_sums.get(), n_pairs, h->d_means.get());
+    CU(cudaGetLastError());
+    return GNSSACQ_OK;
+}
+
 int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xchg) {
     cudaStream_t s = h->stream;
     h->launches = 0;
     auto& xc = h->xc;
     if (xchg && !h->d_comb) return fail(h, GNSSACQ_ERR_STATE, "the multi-GPU exchange needs the comb-row K1 (shared memory too small for this shape)");
     CU(cudaEventRecord(h->ev[1].get(), s));
-    // int16 (acquisition.m:30-32): per-component means of the N*K*M samples, from `scan` (I, Q) pairs at `src`
+    // int16 (acquisition.m:30-32): per-component means of the N*K*M samples
     const double* means = h->cfg.data_precision == 2 ? h->d_means.get() : nullptr;
-    auto launch_means = [&](const void* src, long long scan) -> int {
-        CU(cudaMemsetAsync(h->d_sums.get(), 0, 2 * sizeof(long long), s));
-        sum_int16_kernel<<<296, 256, 0, s>>>((const int16_t*)src, scan, h->d_sums.get());
-        means_kernel<<<1, 1, 0, s>>>(h->d_sums.get(), (long long)h->N * h->K * h->M, h->d_means.get());
-        CU(cudaGetLastError());
-        h->launches += 2;
-        return GNSSACQ_OK;
-    };
+    const long long n_pairs = (long long)h->N * h->K * h->M;
     if (h->d_comb) {
         const int bps = h->cfg.data_type * h->cfg.data_precision;
         const int rows = h->N / 16, tiles = (rows + kCombTM - 1) / kCombTM;
@@ -516,7 +519,8 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
         // from the comb copy, not `d_if`: on a non-root shard that is the root's buffer (see comb_kernel).
         // [K*M*16 rows][pitch bytes], one (I, Q) pair per 4 bytes; the pad bytes are zero (memset at create, never written)
         if (means) {
-            if (int rc = launch_means(h->d_comb.get(), (long long)h->K * h->M * 16 * h->comb_pitch / 4)) return rc;
+            if (int rc = launch_means(h, h->d_comb.get(), (long long)h->K * h->M * 16 * h->comb_pitch / 4, n_pairs, s)) return rc;
+            h->launches += 2;
         }
         Wipe2Args w2;
         w2.comb = h->d_comb.get();
@@ -532,7 +536,8 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
     } else {
         // (K1 v1 is never used by the multi-GPU exchange: `d_if` is this handle's own, complete block)
         if (means) {
-            if (int rc = launch_means(d_if, (long long)h->N * h->K * h->M)) return rc;
+            if (int rc = launch_means(h, d_if, n_pairs, n_pairs, s)) return rc;
+            h->launches += 2;
         }
         WipeArgs wa;
         wa.raw = d_if;
@@ -546,8 +551,7 @@ int enqueue(gnssacq_handle* h, const void* d_if, gnssacq_result* d_out, bool xch
         wa.fs_hz = h->cfg.fs_hz;
         wa.means = means;
         wa.x = h->d_x.get();
-        if (h->NF == h->N) CU(h->ops->launch_wipe(wa, (int)h->base_freq.size() * h->K, s));
-        else CU(h->ops->launch_wipe_pad(wa, (int)h->base_freq.size() * h->K, s));
+        CU(h->ops->launch_wipe(wa, (int)h->base_freq.size() * h->K, s));
         h->launches += 1;
     }
     CU(cudaEventRecord(h->ev[2].get(), s));
@@ -1136,10 +1140,7 @@ int gnssacq_fine_frequency(gnssacq_handle* h, const void* if_long, size_t nbytes
     const double* means = nullptr;
     if (c.data_precision == 2) {                                                // acquisition.m:92-94
         const long long pairs = (long long)(L + 1) * N;
-        CU(cudaMemsetAsync(h->d_sums.get(), 0, 2 * sizeof(long long), s));
-        sum_int16_kernel<<<296, 256, 0, s>>>((const int16_t*)d_raw, pairs, h->d_sums.get());
-        means_kernel<<<1, 1, 0, s>>>(h->d_sums.get(), pairs, h->d_means.get());
-        CU(cudaGetLastError());
+        if (int rc = launch_means(h, d_raw, pairs, pairs, s)) return rc;
         means = h->d_means.get();
     }
     for (int first = 0; first < n_sv; first += chunk) {

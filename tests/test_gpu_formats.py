@@ -4,8 +4,8 @@ stage, the re-acquisition sweeps and the peer-memory exchange with both formats.
 
 The format decides which code runs: comb_kernel and wipe2_kernel branch on the bytes per sample (1 real int8, 2 int8
 I/Q, 4 int16 I/Q), the comb pitch and wipe2's staging depend on them and on Q, and the one shipped shape whose
-staging does not fit in shared memory (Q = 29, 4 CTAs x 512 threads, int16, 2-ms fold) runs the older K1
-(wipe_kernel) instead."""
+staging does not fit in shared memory (Q = 29, 4 CTAs x 512 threads, int16, 2-ms fold) runs the gather K1
+(wipe_pad_kernel) instead."""
 import math
 
 import numpy as np
@@ -104,7 +104,7 @@ def test_every_format_on_every_engine_cell_by_cell(n, fmt, coh_ms):
                 assert_same_argmax(got, w, f"{what} PRN {prn}")
         assert_rows_match(rows, ref, what=what)
     # K1 is comb_kernel + wipe2_kernel (2 launches) wherever wipe2's staging fits in 227 KB of shared memory; the one
-    # shipped shape where it does not (233 728 B) runs wipe_kernel (1 launch).  The last variant of each N is a comb one.
+    # shipped shape where it does not (233 728 B) runs wipe_pad_kernel (1 launch).  The last variant of each N is a comb one.
     no_comb = (n, fmt, coh_ms) == (58000, "iq16", 2)
     comb = launches[VARIANTS[n][-1]]
     assert launches == {v: comb - int(no_comb and v[:2] == (4, 512)) for v in launches}
@@ -219,7 +219,7 @@ def test_peer_exchange_with_both_formats(fmt, plan, world):
 def test_peer_exchange_refuses_the_shape_without_comb_rows():
     """The exchange pulls the IF block with comb_kernel, which the Q = 29 / 4 x 512 / int16 / 2-ms shape does not run:
     making such a handle a root is refused (GNSSACQ_ERR_STATE) and so is a step, before anything is launched that
-    another shard could wait on.  The handle itself still searches, with wipe_kernel."""
+    another shard could wait on.  The handle itself still searches, with wipe_pad_kernel."""
     n, fmt = 58000, "iq16"
     file, signal, acq = grid(n, fmt)
     raw_b = make_block(n, fmt, 2 * K)

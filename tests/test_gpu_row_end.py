@@ -1,9 +1,11 @@
 """The row end of the search (K3) on every engine (`-m gpu`; the geometry port runs on the CPU).
 
-K3 is written three times: in search_kernel (exchange 1), search_kernel_l2x (2) and search_kernel_coop (3).  Each copy
-has its own peak scan over its CTA's column slice, its own +-(w-1) window sum clipped at lags 0 and N-1, and its own
-cross-CTA reduction.  The cooperative kernel has two scans: the debug scan (keep_surface: cell by cell, GeoX::valid)
-and the product scan (float4 loads, `vm >= bv` pruning, padding columns read as exact zeros).  This file checks:
+K3 runs in search_kernel (exchange 1), search_kernel_l2x (2) and search_kernel_coop (3).  All three call one peak scan
+over their CTA's column slice (row_scan) and one +-(w-1) window sum clipped at lags 0 and N-1 (window_sum), each over
+its accumulator layout: columns of Geo / Split for exchanges 1 and 2, of GeoX / SplitX for exchange 3.  Exchanges 1 and
+2 share their cross-CTA reduction (cluster_row_end); exchange 3 has its own.  The cooperative kernel has two scans:
+the debug scan (keep_surface: row_scan, cell by cell, GeoX::valid) and the product scan (float4 loads, `vm >= bv`
+pruning, padding columns read as exact zeros).  This file checks:
 
 - a NumPy port of Geo / GeoX / Split / SplitX (csrc/gnss_engine.h), on the CPU against the header itself, built with
   g++.  The GPU tests take their lags from the port;
